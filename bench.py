@@ -68,7 +68,30 @@ def parse():
                     help="P5: edges sorted by their later pose (as g2o files list them) or the "
                          "loop closures in random order (worst case for locality)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to "
+                         "DIR/<name>.npy (float64): cost, residuals, gradient, jacobian; arrays "
+                         f"longer than {DUMP_SAMPLE} values as a fixed seeded sample whose "
+                         "positions go to DIR/<name>_index.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_SAMPLE = 1 << 20   # values kept per array: 3 arrays and their positions stay under 64 MB
+
+
+def dump_outputs(path, cost, arrays):
+    """Writes cost and each of `arrays` as float64 .npy files under path.  The sample positions
+    depend only on an array's length, so two runs with the same arguments write the same ones."""
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "cost.npy"), np.array([cost], dtype=np.float64))
+    for name, a in arrays.items():
+        idx = np.arange(a.size) if a.size <= DUMP_SAMPLE else np.sort(
+            np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a[idx], dtype=np.float64))
+        np.save(os.path.join(path, name + "_index.npy"), idx.astype(np.float64))
 
 
 class ClockSampler:
@@ -194,10 +217,11 @@ def time_cpu(spec, max_blocks, steps, warmup, fmt=0):
     times = []
     for _ in range(max(1, steps)):
         t0 = time.perf_counter()
-        ok, *_ = op.evaluate(x, num_threads=cores)
+        ok, cost, r, g, j = op.evaluate(x, num_threads=cores)
         times.append(time.perf_counter() - t0)
         assert ok
     per_step = float(np.mean(times))
+    outputs = (cost, {"residuals": r, "gradient": g, "jacobian": j[:op.num_jacobian_values]})
     return {"value": op.num_residual_blocks / per_step, "unit": "residual blocks/s",
             "cores": cores, "kind": "port",
             "build": "oracle/oracle_eval.cc, g++ -O3 -march=native, std::thread static partition",
@@ -205,7 +229,8 @@ def time_cpu(spec, max_blocks, steps, warmup, fmt=0):
                        f"first {op.num_residual_blocks} of {spec.num_rb} residual blocks "
                        f"(whole problem's parameter blocks)") +
                       f", full Evaluate, mean of {len(times)} calls after {max(1, warmup)} warm-up",
-            "ms_per_step": per_step * 1e3, "best_ms": float(min(times)) * 1e3}
+            "ms_per_step": per_step * 1e3, "best_ms": float(min(times)) * 1e3,
+            "outputs": outputs}
 
 
 def run_reference(args):
@@ -217,6 +242,8 @@ def run_reference(args):
     # (L: ~3 s per step on 16 threads).
     steps, warmup = args.steps, args.warmup
     cpu = time_cpu(spec, args.cpu_sample_blocks, steps, warmup, WORKLOADS[args.workload]["fmt"])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *cpu["outputs"])
     line = {
         "impl": "reference", "metric": METRIC,
         "value": cpu["value"], "unit": "residual blocks/s", "n_gpus": args.gpus,
@@ -288,6 +315,8 @@ def run_ours(args):
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: there is no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of one GPU: run it with --gpus 1")
     torch.cuda.set_device(local_rank)
     w = WORKLOADS[args.workload]
 
@@ -371,6 +400,12 @@ def run_ours(args):
     wall_e2e = max_over_ranks(time.perf_counter() - t0)
     e2e_engine_ms = cp.timing()["e2e_ms"]
     clocks = sampler.stop()
+    if args.dump_outputs:
+        # The last timed step: Evaluator::Evaluate into the caller's host buffers, at the state
+        # the device-resident steps evaluated.
+        dump_outputs(args.dump_outputs, cost, {
+            "residuals": residuals.array, "gradient": gradient.array,
+            "jacobian": cp.jacobian_values[:cp.num_jacobian_values]})
     # ---- the candidate-step evaluation of the minimizer (cost only), device time
     cost_only_ms = []
     for _ in range(max(3, args.warmup) + 5):

@@ -150,23 +150,39 @@ struct ResidualType {
 };
 
 // Sums the per-thread-block cost partials in a fixed order (one block, tree in
-// shared memory) and writes the total next to the gradient.
+// shared memory), adds the m per-chunk costs of a chunked launch, also in a fixed order, and
+// writes the total next to the gradient.  Launched with kReduceCostThreads threads; the
+// per-thread-block partials are summed by the first 256 of them.
 // out[1] = the evaluation status as a double, so that it travels through the same sum over
 // the ranks as the cost: every rank then returns the same verdict (a functor failing on one
 // rank fails the whole Evaluate, like the CPU evaluator's all-or-nothing contract).
-__global__ void ReduceCostKernel(const double* __restrict__ partials, int n, double* out,
-                                 const int32_t* __restrict__ status) {
+constexpr int kReduceCostThreads = 1024;
+__global__ void __launch_bounds__(kReduceCostThreads)
+ReduceCostKernel(const double* __restrict__ partials, int n, const double* __restrict__ chunk_costs,
+                 int m, double* out, const int32_t* __restrict__ status) {
   __shared__ double sm[256];
+  __shared__ double chunk_sm[kReduceCostThreads];
+  const int tid = threadIdx.x;
+  if (tid < 256) {
+    double acc = 0.0;
+    for (int i = tid; i < n; i += 256) acc += partials[i];
+    sm[tid] = acc;
+  }
+  // ~30 k chunks on the largest problems: eight loads in flight per thread
   double acc = 0.0;
-  for (int i = threadIdx.x; i < n; i += 256) acc += partials[i];
-  sm[threadIdx.x] = acc;
+#pragma unroll 8
+  for (int i = tid; i < m; i += kReduceCostThreads) acc += chunk_costs[i];
+  chunk_sm[tid] = acc;
   __syncthreads();
-  for (int s = 128; s > 0; s >>= 1) {
-    if (threadIdx.x < s) sm[threadIdx.x] += sm[threadIdx.x + s];
+  for (int s = kReduceCostThreads / 2; s > 0; s >>= 1) {
+    if (tid < s) {
+      chunk_sm[tid] += chunk_sm[tid + s];
+      if (s < 256) sm[tid] += sm[tid + s];
+    }
     __syncthreads();
   }
-  if (threadIdx.x == 0) {
-    out[0] = sm[0];
+  if (tid == 0) {
+    out[0] = m > 0 ? sm[0] + chunk_sm[0] : sm[0];
     out[1] = *status ? 1.0 : 0.0;
   }
 }
@@ -876,6 +892,7 @@ struct cb200_engine {
   DeviceBuffer<double> d_state, d_plus, d_residuals, d_jacobian, d_gradcost, d_cost_partials;
   DeviceBuffer<int32_t> d_pb_table, d_status;
   int32_t total_cost_partials = 0;
+  int32_t chunk_cost_capacity = 0;  // per-chunk cost slots, after the total_cost_partials ones
 
   // pinned scalars: [cost, status]
   double* h_scalars = nullptr;
@@ -1072,6 +1089,12 @@ int cb200_engine_set_shard(cb200_engine* e, int32_t rank, int32_t world_size) {
   e->world = world_size;
   return CB200_OK;
 }
+
+// Chunk walk instead of the grid stride for large types (measured on B200, BAL L: 1.774 ms with
+// chunks of 992 blocks against 1.813 ms; chunks must stay >= ~16 per warp of the persistent
+// grid - 148 SMs x 12 warps - or the tail costs more than the walk gains).
+constexpr int32_t kUniformChunkBlocks = 992;
+constexpr int32_t kUniformChunkMinBlocks = 16 * 148 * 12 * 512;
 
 int cb200_engine_finalize(cb200_engine* e) {
   NvtxRange nvtx_range("cb200_engine_finalize");
@@ -1438,7 +1461,13 @@ int cb200_engine_finalize(cb200_engine* e) {
   e->gradcost = e->d_gradcost.ptr;
   if (e->peer_plan && !e->chunk_table.empty())
     CB200_CUDA(e, e->d_chunks.Upload(e->chunk_table, e->stream));
-  CB200_CUDA(e, e->d_cost_partials.Resize(static_cast<size_t>(e->total_cost_partials) + 1));
+  // the largest chunk count one launch can have: the exchange plan's chunks or uniform ones
+  e->chunk_cost_capacity = static_cast<int32_t>(e->chunk_table.size() / 4);
+  for (ResidualType* t : e->types)
+    e->chunk_cost_capacity = std::max(e->chunk_cost_capacity,
+                                      (t->n_local + kUniformChunkBlocks - 1) / kUniformChunkBlocks);
+  CB200_CUDA(e, e->d_cost_partials.Resize(static_cast<size_t>(e->total_cost_partials) +
+                                          e->chunk_cost_capacity + 1));
   CB200_CUDA(e, e->d_status.Resize(2));  // [failure flag, chunk counter of the chunked kernel]
   CB200_CUDA(e, cudaStreamSynchronize(e->stream));
   // Layout arrays were consumed.
@@ -1541,12 +1570,6 @@ int cb200_engine_comm_init(cb200_engine* e, const void* unique_id, int32_t rank,
 }
 
 // Shared by the host-pointer and device-pointer entry points.
-// Chunk walk instead of the grid stride for large types (measured on B200, BAL L: 1.774 ms with
-// chunks of 992 blocks against 1.813 ms; chunks must stay >= ~16 per warp of the persistent
-// grid - 148 SMs x 12 warps - or the tail costs more than the walk gains).
-constexpr int32_t kUniformChunkBlocks = 992;
-constexpr int32_t kUniformChunkMinBlocks = 16 * 148 * 12 * 512;
-
 static int EvaluateOnDevice(cb200_engine* e, uint32_t flags, bool want_r, bool want_g,
                             bool want_j) {
   cudaStream_t s = e->stream;
@@ -1587,6 +1610,7 @@ static int EvaluateOnDevice(cb200_engine* e, uint32_t flags, bool want_r, bool w
   CB200_CUDA(e, cudaEventRecord(e->ev[1], s));
   int launches = 0;
   bool pushed_by_kernel = false;
+  int32_t chunk_costs = 0;  // chunks of this evaluation's chunked launch
   for (ResidualType* t : e->types) {
     if (t->n_local == 0) continue;
     cb200_launch_args a{};
@@ -1627,10 +1651,13 @@ static int EvaluateOnDevice(cb200_engine* e, uint32_t flags, bool want_r, bool w
     std::memcpy(a.jacobian_step, t->jacobian_step, sizeof(a.jacobian_step));
     // The chunked variant exists for the plain all-outputs kernel over affine tables (the
     // same test as in the launch thunk); otherwise PushExclusiveKernel below does the copies.
+    // One chunked launch per evaluation at most: the chunk counter (status[1]) and the chunk
+    // cost slots serve one launch.
     constexpr uint32_t kAffinePlain =
         CB200_AFFINE_RESIDUAL | CB200_AFFINE_JACOBIAN | CB200_AFFINE_DELTA_IS_STATE;
-    if (peer && t->desc.supports_chunks && e->d_chunks.ptr && t->plain && !a.crs && want_r &&
-        want_j && a.apply_loss_function && (t->affine & kAffinePlain) == kAffinePlain &&
+    if (chunk_costs == 0 && peer && t->desc.supports_chunks && e->d_chunks.ptr && t->plain &&
+        !a.crs && want_r && want_j && a.apply_loss_function &&
+        (t->affine & kAffinePlain) == kAffinePlain &&
         // (measured on B200: with two ranks the copies issued from inside the kernel slow it
         // by more than the separate push costs - 1.15 against 1.05 ms of device time on BAL
         // L - while from four ranks on the fused form wins: 0.37 against 0.55 ms on eight)
@@ -1642,12 +1669,16 @@ static int EvaluateOnDevice(cb200_engine* e, uint32_t flags, bool want_r, bool w
       pushed_by_kernel = true;
     }
     // Large single-type problems without in-kernel copies: uniform chunks (see chunk_blocks).
-    if (!a.chunks && t->desc.supports_chunks && t->plain && !a.crs && want_r && want_j && want_g &&
-        a.apply_loss_function && (t->affine & kAffinePlain) == kAffinePlain &&
+    if (chunk_costs == 0 && !a.chunks && t->desc.supports_chunks && t->plain && !a.crs && want_r &&
+        want_j && want_g && a.apply_loss_function && (t->affine & kAffinePlain) == kAffinePlain &&
         t->n_local >= kUniformChunkMinBlocks && !getenv("CB200_NO_CHUNKED_KERNEL")) {
       a.chunk_blocks = kUniformChunkBlocks;
       a.num_chunks = (t->n_local + kUniformChunkBlocks - 1) / kUniformChunkBlocks;
       a.num_peers = 0;
+    }
+    if (a.num_chunks > 0) {
+      a.chunk_cost_offset = e->total_cost_partials - t->cost_partial_offset;
+      chunk_costs = a.num_chunks;
     }
     const int err = t->desc.launch(&a, s);
     if (err != 0)
@@ -1657,8 +1688,10 @@ static int EvaluateOnDevice(cb200_engine* e, uint32_t flags, bool want_r, bool w
   }
   CB200_CUDA(e, cudaEventRecord(e->ev[2], s));
   // [gradient | cost | failed]: the last two slots are written here
-  ReduceCostKernel<<<1, 256, 0, s>>>(e->d_cost_partials.ptr, e->total_cost_partials,
-                                     e->gradcost + ne, e->d_status.ptr);
+  ReduceCostKernel<<<1, kReduceCostThreads, 0, s>>>(
+      e->d_cost_partials.ptr, e->total_cost_partials,
+      e->d_cost_partials.ptr + e->total_cost_partials, chunk_costs, e->gradcost + ne,
+      e->d_status.ptr);
   ++launches;
   if (peer) {
     if (!pushed_by_kernel && e->exclusive_length > 0) {

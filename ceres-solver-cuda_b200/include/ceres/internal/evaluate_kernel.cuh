@@ -1526,6 +1526,15 @@ __global__ void __launch_bounds__(
     parity_cur = parity_issue;
 
     if constexpr (kChunked) {
+      // Last tile of a chunk: the chunk's cost goes to a slot of its own (summed in chunk
+      // order by the engine, whichever warp drew the chunk).
+      if (warp_rb + 32 >= limit) {
+        double chunk_cost = cost_sum;
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) chunk_cost += __shfl_down_sync(0xffffffffu, chunk_cost, d);
+        if (lane == 0) a.cost_partials[a.chunk_cost_offset + c0] = chunk_cost;
+        cost_sum = 0.0;
+      }
       // Last tile of a chunk: its exclusive gradient range is final (no other chunk, on
       // any rank, adds to it).  Make this warp's reductions visible, then copy the range
       // into every other rank's gradient buffer; meanwhile the other warps of this SM keep
@@ -1608,7 +1617,8 @@ __global__ void __launch_bounds__(
   if (!all_ok) *a.status = 1;
 
   // Cost: warp shuffle, then one partial per CTA (summed in a fixed order by the
-  // engine, so the cost is reproducible run to run for a given grid).
+  // engine, so the cost is reproducible run to run for a given grid).  Chunked: zero, every
+  // chunk's cost is in its own slot already.
   double c = cost_sum;
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) c += __shfl_down_sync(0xffffffffu, c, d);
@@ -1713,7 +1723,8 @@ cb200_residual_type MakeResidualType() {
   t.functor_size = static_cast<int32_t>(sizeof(Functor));
   t.loss_size = static_cast<int32_t>(sizeof(Loss));
   t.threads_per_block = kEvaluateThreads;
-  t.supports_chunks = CB200_KERNEL_CHUNKED_EXCHANGE;
+  // (the chunked variant is one of the all-outputs specialisations)
+  t.supports_chunks = CB200_KERNEL_CHUNKED_EXCHANGE && CB200_KERNEL_SPECIALISE_ALL_OUTPUTS;
   t.launch = &LaunchEvaluate<Functor, Loss, kRes, Ns...>;
   t.normal_product = &LaunchNormalProduct<kRes, Ns...>;
   return t;

@@ -138,7 +138,10 @@ typedef struct cb200_launch_args {
    * chunk_blocks residual blocks (a multiple of 32), nothing copied - on large problems the
    * walk itself is ~2 % faster than the grid stride (profiles/r2_kbench_variants.txt). */
   int32_t chunk_blocks;
-  int32_t reserved1;
+  /* Both chunked forms: the cost of chunk c goes to cost_partials[chunk_cost_offset + c] and
+   * the per-thread-block entries hold zero, so the sum of the entries in order does not depend
+   * on which warp drew which chunk. */
+  int32_t chunk_cost_offset;
   double* peer_gradient[CB200_MAX_PEERS];
   /* A copy of the loss object when the type has exactly one (loss_index == NULL) and it fits:
    * kernel arguments live in the constant bank, so the kernel reads the loss parameters as

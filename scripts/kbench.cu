@@ -143,9 +143,12 @@ int main(int argc, char** argv) {
       for (int q = 0; q < a.num_peers; ++q) CK(cudaMalloc(&a.peer_gradient[q], 8 * state.size()));
     }
   }
+  // chunked: one cost slot per chunk after the per-thread-block ones
+  const int cost_slots = grid_max + a.num_chunks;
+  a.chunk_cost_offset = grid_max;
   double *res, *jac, *grad, *cp; int* status;
   CK(cudaMalloc(&res, 16 * (size_t)n)); CK(cudaMalloc(&jac, 192 * (size_t)n));
-  CK(cudaMalloc(&grad, 8 * state.size())); CK(cudaMalloc(&cp, 8 * (size_t)grid_max)); CK(cudaMalloc(&status, 8));
+  CK(cudaMalloc(&grad, 8 * state.size())); CK(cudaMalloc(&cp, 8 * (size_t)cost_slots)); CK(cudaMalloc(&status, 8));
   CK(cudaMemset(status, 0, 8));
   a.residuals = res; a.jacobian_values = jac; a.gradient = grad; a.cost_partials = cp; a.status = status;
   cudaStream_t s; CK(cudaStreamCreate(&s));
@@ -187,7 +190,7 @@ int main(int argc, char** argv) {
                 argc > 6 ? argv[6] : "", nsum / reps, nbest, 192.0 * n / (nsum / reps) / 1e6, ys, ya);
   }
   int st; CK(cudaMemcpy(&st, status, 4, cudaMemcpyDeviceToHost));
-  std::vector<double> part(grid_max); CK(cudaMemcpy(part.data(), cp, 8 * (size_t)grid_max, cudaMemcpyDeviceToHost));
+  std::vector<double> part(cost_slots); CK(cudaMemcpy(part.data(), cp, 8 * (size_t)cost_slots, cudaMemcpyDeviceToHost));
   double cost = 0; for (double v : part) cost += v;
   {
     std::vector<double> gh(state.size()), jh(1 << 16);
