@@ -1422,7 +1422,6 @@ int cb200_engine_finalize(cb200_engine* e) {
       t->affine = (res_affine ? CB200_AFFINE_RESIDUAL : 0u) |
                   (jac_affine ? CB200_AFFINE_JACOBIAN : 0u) |
                   (delta_is_state ? CB200_AFFINE_DELTA_IS_STATE : 0u);
-      if (getenv("CB200_NO_AFFINE")) t->affine = 0;  // A/B switch: always read the tables
     }
     if (e->planning) continue;
     CB200_CUDA(e, t->d_pb.Upload(pb, e->stream));

@@ -52,10 +52,7 @@
 namespace ceres {
 namespace internal {
 
-#ifndef CB200_EVALUATE_THREADS
-#define CB200_EVALUATE_THREADS 128
-#endif
-constexpr int kEvaluateThreads = CB200_EVALUATE_THREADS;
+constexpr int kEvaluateThreads = 128;  // threads per CTA (measured: see ResidentCtas)
 // internal/ceres/array_utils.h: the value autodiff leaves in outputs a functor
 // did not write; evaluations containing it are invalid.
 constexpr double kImpossibleValue = 1e302;
@@ -73,12 +70,6 @@ struct BlockDims {
     for (int i = 0; i < j; ++i) o += Size(i);
     return o;
   }
-  // sum over the blocks before j of their size rounded up to odd (shared-memory pitch)
-  __host__ __device__ static constexpr int PitchBefore(int j) {
-    int o = 0;
-    for (int i = 0; i < j; ++i) o += Size(i) | 1;
-    return o;
-  }
   __host__ __device__ static constexpr int MaxSize() {
     int m = 0;
     for (int i = 0; i < kNumBlocks; ++i) m = Size(i) > m ? Size(i) : m;
@@ -87,14 +78,6 @@ struct BlockDims {
   // 16-byte chunks of the aligned window that contains block j whether its first double
   // sits at an even or an odd offset of the state vector.
   __host__ __device__ static constexpr int WindowChunks(int j) { return Size(j) / 2 + 1; }
-  __host__ __device__ static constexpr int ChunksBefore(int j) {
-    int o = 0;
-    for (int i = 0; i < j; ++i) o += WindowChunks(i);
-    return o;
-  }
-  // chunks per thread; odd, so that the 16-byte copies of 8 consecutive threads (one
-  // shared-memory wavefront) fall into distinct banks
-  __host__ __device__ static constexpr int RowChunks() { return ChunksBefore(kNumBlocks) | 1; }
   // Cooperative gather: a lane's window of block j occupies WindowPitch(j) chunks, odd, so
   // that the owner's reads (lane stride = pitch * 16 bytes) spread over the banks: an even
   // pitch of 2 or 4 chunks puts 32 lanes on 2 or 4 bank groups (measured on the pose graph
@@ -270,62 +253,6 @@ __device__ __forceinline__ void CpAsyncWait() {
   asm volatile("cp.async.wait_group %0;" ::"n"(kPending) : "memory");
 }
 
-// Tuning switches (compile-time; scripts/kbench.cu builds the kernel with several
-// settings to measure each on the GPU).
-#ifndef CB200_KERNEL_FMA_CHECK
-#define CB200_KERNEL_FMA_CHECK 1      // finite check: 1 = FMA chain (FP64 pipe), 0 = integer max
-#endif
-#ifndef CB200_KERNEL_FMA_CHECK_CHAINS
-#define CB200_KERNEL_FMA_CHECK_CHAINS 1
-#endif
-#ifndef CB200_KERNEL_SPECIALISE_ALL_OUTPUTS
-#define CB200_KERNEL_SPECIALISE_ALL_OUTPUTS 1  // extra instantiations for the all-outputs call
-#endif
-#ifndef CB200_KERNEL_STAGE_GRADIENT
-#define CB200_KERNEL_STAGE_GRADIENT 1 // warp-staged, sector-coalesced gradient reductions
-#endif
-#ifndef CB200_KERNEL_STAGE_GRADIENT_MIN_SIZE
-#define CB200_KERNEL_STAGE_GRADIENT_MIN_SIZE 1  // smaller blocks add their sums directly
-#endif
-#ifndef CB200_KERNEL_STAGE_JACOBIAN
-#define CB200_KERNEL_STAGE_JACOBIAN 1 // warp-staged, fully coalesced Jacobian stores
-#endif
-#ifndef CB200_KERNEL_BULK_STORE
-#define CB200_KERNEL_BULK_STORE 1     // staged cells leave through TMA bulk copies (UBLKCP)
-#endif
-#ifndef CB200_KERNEL_GRADIENT_DESTINATIONS
-// 1: the lane that stages its gradient sums also stages the destination of every element, so
-// a reduction round is two shared loads, one 64-bit multiply-add for the address and the
-// red (4 instructions); 0: destinations are staged per lane and every round recomputes the
-// (row, column) of its element (9 instructions, measured: 111 of the BAL kernel's 1184
-// instructions per tile were address arithmetic of the rounds).
-#define CB200_KERNEL_GRADIENT_DESTINATIONS 1
-#endif
-#ifndef CB200_KERNEL_GATHER
-// How a warp's 32 residual blocks fetch their parameter blocks into shared memory:
-// 0 = warp-cooperative, 8-byte copies, consecutive lanes on consecutive doubles of a block;
-// 1 = every thread copies its own blocks, 16-byte pieces of the aligned window;
-// 2 = warp-cooperative, 16-byte pieces of the aligned windows.
-#define CB200_KERNEL_GATHER 2
-#endif
-#ifndef CB200_KERNEL_PARAM_READ128
-#define CB200_KERNEL_PARAM_READ128 1  // gather 2: the owner reads its windows with 16-byte loads
-#endif
-#ifndef CB200_KERNEL_EARLY_PREFETCH
-// 1: parameters and functor are double-buffered and the copies for block k+1 are issued
-// before block k is computed; 0: single-buffered, issued after block k's last functor call.
-#define CB200_KERNEL_EARLY_PREFETCH 1
-#endif
-#ifndef CB200_KERNEL_CHUNKED_EXCHANGE
-#define CB200_KERNEL_CHUNKED_EXCHANGE 1  // instantiate the chunked (multi-rank) kernel variant
-#endif
-#ifndef CB200_KERNEL_PEER_BULK_STORE
-#define CB200_KERNEL_PEER_BULK_STORE 1  // chunked kernel: exclusive ranges leave through TMA bulk stores
-#endif
-#ifndef CB200_KERNEL_SEGMENTED_GRADIENT
-#define CB200_KERNEL_SEGMENTED_GRADIENT 1  // warp-shuffle pre-reduction of long same-block runs
-#endif
-
 // ---- TMA bulk store shared -> global (cp.async.bulk): one instruction moves a
 // warp's whole run of Jacobian cells; no LDS / STG / address arithmetic per element.
 __device__ __forceinline__ void FenceProxyAsyncShared() {
@@ -351,11 +278,12 @@ __host__ __device__ constexpr int MaxInt(int a, int b) { return a > b ? a : b; }
 
 // Accumulates evidence of a non-finite value; Bad() is true iff one was seen.
 struct FiniteCheck {
-#if CB200_KERNEL_FMA_CHECK
-  // Every accumulator stays 0 iff its values are finite (0 * Inf = NaN).  The number of
-  // independent chains is a tuning knob; one chain measured fastest on B200 (BAL L:
-  // 2.28 ms against 2.32 ms with four - the extra accumulators cost registers).
-  static constexpr int kChains = CB200_KERNEL_FMA_CHECK_CHAINS;
+  // Every accumulator stays 0 iff its values are finite (0 * Inf = NaN).  One chain measured
+  // fastest on B200 (BAL L: 2.28 ms against 2.32 ms with four - the extra accumulators cost
+  // registers).  The chain array and its counter stay although kChains is 1: where a
+  // caller's loop is not fully unrolled, a plain scalar accumulator changes the kernel's
+  // registers and stack frame (the pose-graph cost kernels, test functors), unmeasured.
+  static constexpr int kChains = 1;
   double acc[kChains] = {};
   int next = 0;  // folds to a constant once the callers' loops are unrolled
   __device__ __forceinline__ void Add(double x) {
@@ -368,13 +296,6 @@ struct FiniteCheck {
     for (int k = 1; k < kChains; ++k) sum += acc[k];
     return !(sum == 0.0);
   }
-#else
-  unsigned worst = 0;  // max of the high words with the sign shifted out
-  __device__ __forceinline__ void Add(double x) {
-    worst = max(worst, static_cast<unsigned>(__double2hiint(x)) << 1);
-  }
-  __device__ __forceinline__ bool Bad() const { return worst >= 0xffe00000u; }
-#endif
 };
 
 // Loss classes may declare `static constexpr bool kNonPositiveCurvature = true` (rho'' <= 0
@@ -413,10 +334,10 @@ template <int kRes, int... Ns>
 struct PassPlan {
   using Dims = BlockDims<Ns...>;
   static constexpr int kNB = Dims::kNumBlocks;
-#ifndef CB200_SINGLE_PASS_LIMIT
-#define CB200_SINGLE_PASS_LIMIT 40  // live output doubles (residuals x parameters) up to which one pass is used
-#endif
-  static constexpr bool kSinglePass = kRes * Dims::kNumParameters <= CB200_SINGLE_PASS_LIMIT;
+  // Live output doubles (residuals x parameters) up to which one pass is used.  BAL (2 x 12)
+  // in two passes, i.e. a limit of 20, measured 2.09 ms against 1.84 ms on B200 (DESIGN.md 3.1).
+  static constexpr int kSinglePassLimit = 40;
+  static constexpr bool kSinglePass = kRes * Dims::kNumParameters <= kSinglePassLimit;
   static constexpr int kMaxWidth = Dims::MaxSize() > 8 ? Dims::MaxSize() : 8;
   // pass index of block j: greedy grouping of consecutive blocks up to kMaxWidth lanes
   __host__ __device__ static constexpr int PassOf(int j) {
@@ -484,19 +405,13 @@ __host__ __device__ constexpr int MaxStageDoubles() {
 // 1.98 ms; 4 x 128 (128 registers, no spills) 2.08; 2 x 128 (242 registers) 2.36; 5 x 96 2.16;
 // 3 x 160 2.19; 7 x 64 2.19 - more warps cost the compiler the registers it uses to overlap
 // independent Jet lanes, fewer warps cost latency hiding.  Wide problems get 2 CTAs.
-#ifndef CB200_RESIDENT_CTAS_SMALL
-#define CB200_RESIDENT_CTAS_SMALL 3
-#endif
-#ifndef CB200_RESIDENT_CTAS_COST
-#define CB200_RESIDENT_CTAS_COST 6  // CTAs per SM wanted for the Jet-free variant
-#endif
-#ifndef CB200_RESIDENT_CTAS_TABLES
-#define CB200_RESIDENT_CTAS_TABLES 3  // variants that stage the int tables need more shared memory
-#endif
+constexpr int kResidentCtasSmall = 3;
+constexpr int kResidentCtasCost = 6;    // CTAs per SM wanted for the Jet-free variant
+constexpr int kResidentCtasTables = 3;  // variants that stage the int tables: more shared memory
 __host__ __device__ constexpr int ResidentCtas(int num_residuals, int num_parameters,
                                                bool int_tables = false) {
   return (num_parameters <= 13 && num_residuals <= 3)
-             ? (int_tables ? CB200_RESIDENT_CTAS_TABLES : CB200_RESIDENT_CTAS_SMALL)
+             ? (int_tables ? kResidentCtasTables : kResidentCtasSmall)
              : 2;
 }
 // Dynamic shared memory a CTA may use so that `ctas` of them fit on an SM (228 KB per SM,
@@ -507,21 +422,19 @@ __host__ __device__ constexpr int SmemBudget(int ctas) {
 }
 
 // Shared memory plan of a kernel instantiation.  Per CTA:
-//   [parameters: one row of 16-byte windows per thread][functor slot per thread]
+//   [parameters, two stages: per warp, the 16-byte windows of its 32 blocks]
+//   [functor slot per thread, two stages]
 //   [per-block integer tables, two stages — absent when kInts is false]
 //   [per warp: Jacobian staging | gradient staging]
-// Parameters and functor are single-buffered: the copies for the next residual block are
-// issued after the last functor call of the current one, into the rows just consumed.
+// Parameters, functor and tables are double-buffered: the copies for residual block k+1 are
+// issued at the top of iteration k, into the stage block k-1 used, and land while block k is
+// computed.
 template <typename Functor, bool kInts, int kRes, int... Ns>
 struct SmemPlan {
   using Dims = BlockDims<Ns...>;
   static constexpr int kNB = Dims::kNumBlocks;
   // bytes per thread of one parameter stage
-  static constexpr int kParamBytes =
-      CB200_KERNEL_GATHER == 0 ? Dims::PitchBefore(kNB) * 8
-                               : (CB200_KERNEL_GATHER == 1 ? Dims::RowChunks() * 16
-                                                           : Dims::PitchChunksBefore(kNB) * 16);
-  static constexpr int kStages = CB200_KERNEL_EARLY_PREFETCH ? 2 : 1;
+  static constexpr int kParamBytes = Dims::PitchChunksBefore(kNB) * 16;
   static constexpr bool kFunctorInSmem =
       (sizeof(Functor) % 4 == 0) && (alignof(Functor) <= 16) && (sizeof(Functor) <= 128);
   static constexpr int kFunctorBytes = kFunctorInSmem ? static_cast<int>(sizeof(Functor)) : 0;
@@ -536,9 +449,9 @@ struct SmemPlan {
 
   static constexpr int kParamOffset = 0;
   static constexpr int kParamStageBytes = kParamBytes * kEvaluateThreads;
-  static constexpr int kFunctorOffset = kStages * kParamStageBytes;
+  static constexpr int kFunctorOffset = 2 * kParamStageBytes;
   static constexpr int kFunctorStageBytes = kFunctorSlot * kEvaluateThreads;
-  static constexpr int kIntOffset = kFunctorOffset + kStages * kFunctorStageBytes;
+  static constexpr int kIntOffset = kFunctorOffset + 2 * kFunctorStageBytes;
   static constexpr int kPrefetchRaw = kIntOffset + 2 * kIntStageBytes;
   static constexpr bool kFits = kPrefetchRaw <= 96 * 1024;
   static constexpr int kPrefetchBytes = kFits ? kPrefetchRaw : 0;
@@ -551,19 +464,14 @@ struct SmemPlan {
   // element, its destination in the gradient (an int; -1 = nothing to add).  Within a
   // derivative pass every gradient is out before the first cell is staged, so the gradient
   // staging reuses the Jacobian staging buffer.
-#if CB200_KERNEL_GRADIENT_DESTINATIONS
   static constexpr int kGradientStage = 48 * StagePitch(Dims::MaxSize());
-#else
-  static constexpr int kGradientStage = 32 * StagePitch(Dims::MaxSize()) + 32;
-#endif
   // (several passes: each pass waits for the previous pass's stores to leave the staging
   // region before its own gradient uses it, so the alias holds pass by pass)
   static constexpr bool kGradientAliasesJacobian = kGradientStage <= kJacobianDoubles;
   static constexpr int kGradientDoubles = kGradientAliasesJacobian ? 0 : kGradientStage;
   static constexpr int kWarps = kEvaluateThreads / 32;
   static constexpr bool kStageJacobian =
-      CB200_KERNEL_STAGE_JACOBIAN &&
-      (kPrefetchBytes + kWarps * (kJacobianDoubles + kGradientDoubles) * 8 <= SmemBudget(kCtas));
+      kPrefetchBytes + kWarps * (kJacobianDoubles + kGradientDoubles) * 8 <= SmemBudget(kCtas);
   static constexpr int kGradientOffset =
       (kStageJacobian && !kGradientAliasesJacobian) ? kJacobianDoubles : 0;
   static constexpr int kWarpDoubles =
@@ -578,18 +486,18 @@ struct SmemPlan {
 __host__ __device__ constexpr int VariantCtas(int variant, int resident, int cost_bytes) {
   if (variant != kVariantCost) return resident;
   const int by_smem = (227 * 1024) / (cost_bytes + 1024);
-  const int wanted = CB200_RESIDENT_CTAS_COST;
+  const int wanted = kResidentCtasCost;
   return by_smem < resident ? resident : (by_smem < wanted ? by_smem : wanted);
 }
 
 // One thread evaluates one residual block at a time and walks the type's blocks with a
 // grid stride (persistent CTAs).  Software pipeline per thread:
-//   iteration k:  [state offsets of block k+1 -> registers]
+//   iteration k:  [cp.async parameters + functor (+ int tables) of block k+1 -> other stage]
+//                 [state offsets of block k+2 -> registers]
 //                 [wait for block k's copies] functor of block k from shared memory
-//                 [cp.async parameters + functor (+ int tables) of block k+1 -> shared]
 //                 epilogue of block k (loss, gradient, scatter)
 // so the two dependent global loads (offset, then the gathered parameters) of a block are
-// in flight during the functor and the epilogue of the previous block instead of stalling
+// in flight while the blocks before it are computed instead of stalling
 // the warp (v1 of this kernel: long-scoreboard stalls 7.5 of 15 cycles per issue, FP64 pipe
 // 22% busy; profiles/r1_v1_ncu_summary.txt).  a.state must be 16-byte aligned and followed
 // by at least two doubles of slack (the engine's state buffer is).
@@ -650,16 +558,14 @@ __global__ void __launch_bounds__(
   const int iterations = cta_first < n ? (n - cta_first + stride - 1) / stride : 0;
 
   auto clamp = [&](int rb) { return rb < n ? rb : n - 1; };
-  constexpr int kStages = Smem::kStages;
-  // parameter stage: per-thread rows (gather 1) or one region per warp (gathers 0, 2)
+  // this warp's region of parameter stage `stage`
   auto stage_params = [&](int stage) {
-    double* base = reinterpret_cast<double*>(smem + Smem::kParamOffset +
-                                             (kStages > 1 ? stage : 0) * Smem::kParamStageBytes);
-    return CB200_KERNEL_GATHER == 1 ? base + tid * (Smem::kParamBytes / 8)
-                                    : base + (tid >> 5) * 32 * (Smem::kParamBytes / 8);
+    double* base =
+        reinterpret_cast<double*>(smem + Smem::kParamOffset + stage * Smem::kParamStageBytes);
+    return base + (tid >> 5) * 32 * (Smem::kParamBytes / 8);
   };
   auto stage_functor = [&](int stage) {
-    return smem + Smem::kFunctorOffset + (kStages > 1 ? stage : 0) * Smem::kFunctorStageBytes +
+    return smem + Smem::kFunctorOffset + stage * Smem::kFunctorStageBytes +
            tid * Smem::kFunctorSlot;
   };
   auto stage_ints = [&](int stage) {
@@ -677,57 +583,27 @@ __global__ void __launch_bounds__(
     for (int j = 0; j < kNB; ++j) p |= static_cast<unsigned>(soff[j] & 1) << j;
     return p;
   };
-  // Issues the copies of residual block rb: its parameter blocks (into this thread's row),
-  // its functor, and — table variants — its integers into int stage `stage`.
+  // Issues the copies of residual block rb: its parameter blocks (into its warp's region of
+  // parameter stage `stage`), its functor, and — table variants — its integers.
   auto prefetch = [&](int stage, int rb, const int (&soff)[kNB]) {
     if constexpr (kPrefetch) {
       double* dst = stage_params(stage);
-      if constexpr (CB200_KERNEL_GATHER == 1) {
-        // Every thread copies its own blocks in 16-byte pieces: the aligned window
-        // [start & ~1, ...) of Size/2 + 1 pieces holds the block for either parity of its
-        // start.  The owner reads from (start & 1) on.
+      // The aligned window [start & ~1, ...) of W = Size/2 + 1 16-byte pieces holds a block
+      // for either parity of its start; the owner reads from (start & 1) on.  The warp copies
+      // the 32 windows of argument j as one stream of 32 * W pieces: consecutive lanes fetch
+      // consecutive pieces of a window, so a copy instruction touches a handful of cache lines
+      // instead of 32; shared layout [argument][lane][odd pitch of W | 1 pieces].
 #pragma unroll
-        for (int j = 0; j < kNB; ++j) {
-          const double* __restrict__ src = a.state + (soff[j] & ~1);
+      for (int j = 0; j < kNB; ++j) {
+        const int kW = Dims::WindowChunks(j);  // constant after unrolling
 #pragma unroll
-          for (int c = 0; c < Dims::WindowChunks(j); ++c)
-            CpAsync16(dst + 2 * (Dims::ChunksBefore(j) + c), src + 2 * c);
-        }
-      } else if constexpr (CB200_KERNEL_GATHER == 2) {
-        // The warp copies the 32 windows of argument j as one stream of 32 * W 16-byte
-        // pieces (W = Size/2 + 1): consecutive lanes fetch consecutive pieces of a window,
-        // so a copy instruction touches a handful of cache lines instead of 32; shared
-        // layout [argument][lane][odd pitch of W | 1 pieces].
-#pragma unroll
-        for (int j = 0; j < kNB; ++j) {
-          const int kW = Dims::WindowChunks(j);  // constant after unrolling
-#pragma unroll
-          for (int it = 0; it < kW; ++it) {
-            const int e = it * 32 + lane;
-            const int owner = e / kW;
-            const int c = e - owner * kW;
-            const int so = __shfl_sync(0xffffffffu, soff[j], owner);
-            CpAsync16(dst + 2 * (32 * Dims::PitchChunksBefore(j) + owner * Dims::WindowPitch(j) + c),
-                      a.state + ((so & ~1) + 2 * c));
-          }
-        }
-      } else {
-        // The warp copies its 32 blocks of argument j as one stream of 32 * Size(j)
-        // doubles: consecutive lanes fetch consecutive doubles of a block.  Shared layout
-        // per warp: [argument][lane][pitch], pitch odd (conflict free for the owner).
-#pragma unroll
-        for (int j = 0; j < kNB; ++j) {
-          const int kS = Dims::Size(j);  // constants after unrolling
-          const int kP = kS | 1;
-#pragma unroll
-          for (int it = 0; it < kS; ++it) {
-            const int e = it * 32 + lane;
-            const int owner = e / kS;
-            const int i = e - owner * kS;
-            const int so = __shfl_sync(0xffffffffu, soff[j], owner);
-            CpAsync8(dst + 32 * Dims::PitchBefore(j) + (kP == kS ? e : owner * kP + i),
-                     a.state + (so + i));
-          }
+        for (int it = 0; it < kW; ++it) {
+          const int e = it * 32 + lane;
+          const int owner = e / kW;
+          const int c = e - owner * kW;
+          const int so = __shfl_sync(0xffffffffu, soff[j], owner);
+          CpAsync16(dst + 2 * (32 * Dims::PitchChunksBefore(j) + owner * Dims::WindowPitch(j) + c),
+                    a.state + ((so & ~1) + 2 * c));
         }
       }
       // The int tables of the block (consumed in the epilogue, from shared memory, so
@@ -845,34 +721,31 @@ __global__ void __launch_bounds__(
     const bool warp_valid = warp_rb + 31 < limit;
     const int rb_next = kChunked ? rb1 : rb + stride;
 
-    // The offsets of the next block arrive while this one is computed; its copies are
-    // issued after the last functor call below.
+    // The offsets of the next block arrived during the previous iteration: its copies go to
+    // the other stage now and land while this block is computed.
     int soff_issue[kNB];
 #pragma unroll
     for (int j = 0; j < kNB; ++j) soff_issue[j] = soff_next[j];
     const unsigned parity_issue = parity_of(soff_issue);
-    bool issued = false;
+    // (a lambda called once: inlined as a unit, it keeps the instruction schedule the kernel
+    // was measured with; the same statements written inline make the compiler order the loop
+    // differently, e.g. 32 more instructions and 2 more registers in the affine BAL kernel)
     auto issue_next = [&]() {
-      if (!issued) {
-        // (cooperative gathers overwrite rows other lanes read: the warp must be past them)
-        if constexpr (kPrefetch && kStages == 1 && CB200_KERNEL_GATHER != 1) __syncwarp();
-        prefetch(stage ^ 1, rb_next, soff_issue);
-        // The offsets of block k+2 are fetched right after the copies of block k+1 are
-        // issued: the load then writes the registers the copies just released and is not
-        // needed for a whole iteration.  Fetched before, ptxas keeps the loaded value in a
-        // temporary and moves it into the loop-carried register at once, i.e. it waits for
-        // a load it issued ~40 instructions earlier (one fifth of the kernel's stall
-        // samples, profiles/r2_v10_offset_load_stall.txt).
-        load_offsets(kChunked ? walk_rb(walk) : rb + 2 * stride, soff_next);
-      }
-      issued = true;
+      prefetch(stage ^ 1, rb_next, soff_issue);
+      // The offsets of block k+2 are fetched right after the copies of block k+1 are issued:
+      // the load then writes the registers the copies just released and is not needed for a
+      // whole iteration.  Fetched before, ptxas keeps the loaded value in a temporary and
+      // moves it into the loop-carried register at once, i.e. it waits for a load it issued
+      // ~40 instructions earlier (one fifth of the kernel's stall samples,
+      // profiles/r2_v10_offset_load_stall.txt).
+      load_offsets(kChunked ? walk_rb(walk) : rb + 2 * stride, soff_next);
     };
-    if constexpr (kStages > 1) issue_next();
+    issue_next();
 
     if constexpr (kPrefetch) {
-      // this thread's copies for block k have landed ...
-      if constexpr (kStages > 1) CpAsyncWait<1>(); else CpAsyncWait<0>();
-      if constexpr (CB200_KERNEL_GATHER != 1) __syncwarp();  // ... and its warp's
+      // this thread's copies for block k have landed (block k+1's may be in flight) ...
+      CpAsyncWait<1>();
+      __syncwarp();  // ... and its warp's
     }
 
     // Per-block int tables: from the prefetched stage, computed (affine), or straight
@@ -957,18 +830,6 @@ __global__ void __launch_bounds__(
     const Loss& loss = kInlineLoss ? *reinterpret_cast<const Loss*>(&loss_bytes) : losses[loss_at];
 
     const double* sp = stage_params(stage);
-    auto param = [&](int j, int i) -> double {
-      if constexpr (kPrefetch && CB200_KERNEL_GATHER == 1) {
-        return sp[2 * Dims::ChunksBefore(j) + ((parity_cur >> j) & 1) + i];
-      } else if constexpr (kPrefetch && CB200_KERNEL_GATHER == 2) {
-        return sp[2 * (32 * Dims::PitchChunksBefore(j) + lane * Dims::WindowPitch(j)) +
-                  ((parity_cur >> j) & 1) + i];
-      } else if constexpr (kPrefetch) {
-        return sp[32 * Dims::PitchBefore(j) + lane * (Dims::Size(j) | 1) + i];
-      } else {
-        return __ldg(a.state + soff_cur[j] + i);
-      }
-    };
     const Functor* functor_ptr;
     if constexpr (kPrefetch && Smem::kFunctorInSmem) {
       functor_ptr = reinterpret_cast<const Functor*>(stage_functor(stage));
@@ -978,7 +839,7 @@ __global__ void __launch_bounds__(
     const Functor& functor = *functor_ptr;
 
     double xval[kNP];
-    if constexpr (kPrefetch && CB200_KERNEL_GATHER == 2 && CB200_KERNEL_PARAM_READ128) {
+    if constexpr (kPrefetch) {
       // The owner reads its windows in 16-byte pieces (lane pitch odd in pieces: conflict
       // free, 4 wavefronts per instruction) and picks the doubles by the block's parity; the
       // 8-byte reads at an even lane pitch are two-way bank conflicted (72 wavefronts per tile
@@ -1005,7 +866,8 @@ __global__ void __launch_bounds__(
 #pragma unroll
       for (int j = 0; j < kNB; ++j)
 #pragma unroll
-        for (int i = 0; i < Dims::Size(j); ++i) xval[Dims::Offset(j) + i] = param(j, i);
+        for (int i = 0; i < Dims::Size(j); ++i)
+          xval[Dims::Offset(j) + i] = __ldg(a.state + soff_cur[j] + i);
     }
 
     double res[kRes];
@@ -1018,7 +880,6 @@ __global__ void __launch_bounds__(
 #pragma unroll
       for (int r = 0; r < kRes; ++r) res[r] = kNaN;  // unwritten outputs stay invalid
       ok = CallFunctor<Dims>(functor, xval, res, std::make_index_sequence<kNB>{});
-      issue_next();
       FiniteCheck check;
 #pragma unroll
       for (int r = 0; r < kRes; ++r) check.Add(res[r]);
@@ -1063,7 +924,7 @@ __global__ void __launch_bounds__(
       // the whole L2 round trip - 12 % of the pose-graph kernel's stall samples)
       auto make_store_plan = [&]() {
       if constexpr (kStage) {
-        if (out_jacobian && CB200_KERNEL_BULK_STORE) {
+        if (out_jacobian) {
           if (!crs) {
 #pragma unroll
             for (int j = 0; j < kNB; ++j) {
@@ -1130,9 +991,6 @@ __global__ void __launch_bounds__(
 #pragma unroll
         for (int r = 0; r < kRes; ++r) out[r] = JetT::Filled(kNaN, kNaN);
         ok = CallFunctor<Dims>(functor, x, out, std::make_index_sequence<kNB>{}) && ok;
-        // Parameters and functor of this block are consumed (the last pass re-reads
-        // neither): their rows take the next block's copies.
-        if constexpr (p == Plan::kNumPasses - 1) issue_next();
         if constexpr (p == 0) make_store_plan();
 
         FiniteCheck check;
@@ -1271,31 +1129,31 @@ __global__ void __launch_bounds__(
             // to memory.  Short runs (the 3-10 observations of a BAL point) go out
             // directly: lanes of one red instruction that hit the same sector share one
             // L2 request, which is cheaper than 5 shuffle steps per value.
-            bool head = true;
-            if constexpr (CB200_KERNEL_SEGMENTED_GRADIENT) {
-              const int k_ = (valid && active) ? run_key : -1 - lane;
-              const int prev_key = __shfl_up_sync(0xffffffffu, k_, 1);
-              head = (lane == 0) || (prev_key != k_);
-              const unsigned heads = __ballot_sync(0xffffffffu, head);
-              if (__popc(heads) <= 4) {
+            const int k_ = (valid && active) ? run_key : -1 - lane;
+            const int prev_key = __shfl_up_sync(0xffffffffu, k_, 1);
+            bool head = (lane == 0) || (prev_key != k_);
+            const unsigned heads = __ballot_sync(0xffffffffu, head);
+            if (__popc(heads) <= 4) {
 #pragma unroll
-                for (int c = 0; c < kSize; ++c) g[c] = (valid && ok && active) ? g[c] : 0.0;
-                const unsigned above = lane == 31 ? 0u : (heads & ~((2u << lane) - 1u));
-                const int run_end = above ? __ffs(above) - 1 : 32;
-                WarpSegmentedSum<kSize>(run_end, g, lane);
-              } else {
-                head = true;  // every lane adds its own contribution
-              }
+              for (int c = 0; c < kSize; ++c) g[c] = (valid && ok && active) ? g[c] : 0.0;
+              const unsigned above = lane == 31 ? 0u : (heads & ~((2u << lane) - 1u));
+              const int run_end = above ? __ffs(above) - 1 : 32;
+              WarpSegmentedSum<kSize>(run_end, g, lane);
+            } else {
+              head = true;  // every lane adds its own contribution
             }
             const bool emit = head && valid && ok && active;
             const unsigned emit_mask = __ballot_sync(0xffffffffu, emit);
-            if (CB200_KERNEL_STAGE_GRADIENT && kSize >= CB200_KERNEL_STAGE_GRADIENT_MIN_SIZE &&
-                __popc(emit_mask) >= 12) {
+            if (__popc(emit_mask) >= 12) {
               // Most lanes own a distinct block (the cameras of a BAL warp): stage the
               // per-lane sums and let consecutive lanes add to consecutive addresses, so
-              // one red instruction touches a few sectors instead of 32.
+              // one red instruction touches a few sectors instead of 32.  Each lane also
+              // stages the destination of every element it stages, so a reduction round is
+              // two shared loads, one 64-bit multiply-add for the address and the red (4
+              // instructions); recomputing the (row, column) of the element in every round
+              // took 9 (measured: 111 of the BAL kernel's 1184 instructions per tile were
+              // address arithmetic of the rounds).
               constexpr int kPitch = StagePitch(kSize);
-#if CB200_KERNEL_GRADIENT_DESTINATIONS
               int next = doff;  // destination of the next live column
 #pragma unroll
               for (int c = 0; c < kSize; ++c) {
@@ -1318,42 +1176,6 @@ __global__ void __launch_bounds__(
                   RedAddIf(d >= 0, a.gradient + d, gbuf[it * 32 + lane]);
                 }
               }
-#else
-#pragma unroll
-              for (int c = 0; c < kSize; ++c) gbuf[lane * kPitch + c] = g[c];
-              // destination of every lane's sums (or -1) and, with manifolds, its live
-              // columns: the reduction rounds read them back by row, so a round is two
-              // shared loads, an address and one predicated red
-              obuf[lane] = emit ? doff : -1;
-              if constexpr (kGeneric) obuf[32 + lane] = static_cast<int>(lv);
-              __syncwarp();
-              if (!kGeneric && emit_mask == 0xffffffffu) {
-                // every lane emits (the usual case): straight-line, no per-round branch
-#pragma unroll
-                for (int it = 0; it < kSize; ++it) {
-                  const int e = it * 32 + lane;
-                  const int row = e / kSize;
-                  const int c = e - row * kSize;
-                  RedAdd(a.gradient + (obuf[row] + c),
-                         gbuf[kPitch == kSize ? e : row * kPitch + c]);
-                }
-              } else
-#pragma unroll
-              for (int it = 0; it < kSize; ++it) {
-                const int e = it * 32 + lane;
-                const int row = e / kSize;
-                const int c = e - row * kSize;
-                const int d = obuf[row];
-                const double sum = gbuf[kPitch == kSize ? e : row * kPitch + c];
-                if constexpr (kGeneric) {
-                  const unsigned lr = static_cast<unsigned>(obuf[32 + row]);
-                  RedAddIf(d >= 0 && ((lr >> c) & 1u),
-                           a.gradient + d + __popc(lr & ((1u << c) - 1u)), sum);
-                } else {
-                  RedAddIf(d >= 0, a.gradient + (d + c), sum);
-                }
-              }
-#endif
               __syncwarp();
             } else if (emit) {
               double* __restrict__ dst = a.gradient + doff;
@@ -1547,13 +1369,12 @@ __global__ void __launch_bounds__(
         __threadfence_block();
         __syncwarp();
         const int4 rec = __ldg(chunk_table + c0);
-#if CB200_KERNEL_PEER_BULK_STORE
         // The range goes to the peers through the copy engine (one bulk store per peer and
         // piece, shared -> peer memory over NVLink): stores issued by the lanes themselves sit
         // in the SM's load/store queue until NVLink takes them and hold up every other warp's
-        // memory instructions behind them.  Staged in this tile's parameter rows, which are
+        // memory instructions behind them.  Staged in this tile's parameter stage, which is
         // free until the next iteration's prefetch; 16-byte granularity, odd ends by lane 0/1.
-        if constexpr (kPrefetch && CB200_KERNEL_GATHER != 1) {
+        if constexpr (kPrefetch) {
           const int d0 = rec.z, d1 = rec.w;
           const int a0 = (d0 + 1) & ~1, a1 = d1 & ~1;
           if (lane == 0 && d0 < a0 && d0 < d1) {
@@ -1588,20 +1409,21 @@ __global__ void __launch_bounds__(
             __syncwarp();
             bulk_pending = false;
           }
-        } else
-#endif
-        // four independent loads in flight per lane: the loop is latency bound otherwise
-        for (int i0 = rec.z + lane; i0 < rec.w; i0 += 128) {
-          double v[4];
-#pragma unroll
-          for (int u = 0; u < 4; ++u)
-            v[u] = i0 + 32 * u < rec.w ? __ldcg(a.gradient + i0 + 32 * u) : 0.0;
-#pragma unroll 1
-          for (int q = 0; q < a.num_peers; ++q) {
-            double* __restrict__ dst = a.peer_gradient[q];
+        } else {
+          // (no parameter stage to stage in: the lanes store the range themselves)
+          // four independent loads in flight per lane: the loop is latency bound otherwise
+          for (int i0 = rec.z + lane; i0 < rec.w; i0 += 128) {
+            double v[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u)
-              if (i0 + 32 * u < rec.w) __stcg(dst + i0 + 32 * u, v[u]);
+              v[u] = i0 + 32 * u < rec.w ? __ldcg(a.gradient + i0 + 32 * u) : 0.0;
+#pragma unroll 1
+            for (int q = 0; q < a.num_peers; ++q) {
+              double* __restrict__ dst = a.peer_gradient[q];
+#pragma unroll
+              for (int u = 0; u < 4; ++u)
+                if (i0 + 32 * u < rec.w) __stcg(dst + i0 + 32 * u, v[u]);
+            }
           }
         }
       }
@@ -1677,15 +1499,12 @@ int LaunchEvaluate(const cb200_launch_args* args, void* stream) {
     return LaunchVariant(EvaluateKernel<kVariantCost, false, false, Functor, Loss, kRes, Ns...>, kCostCtas,
                          Computed::kCostBytes, args, s);
   }
-#if CB200_KERNEL_SPECIALISE_ALL_OUTPUTS
   if (all && args->plain && !args->crs) {
-#if CB200_KERNEL_CHUNKED_EXCHANGE
     if ((args->chunks || args->num_chunks > 0) && (args->affine & kAffinePlain) == kAffinePlain)
       return LaunchVariant(
           EvaluateKernel<kVariantPlainAll, true, true, Functor, Loss, kRes, Ns...>, kAffineCtas,
           Computed::kJetBytes, args, s,
           (args->num_chunks + kEvaluateThreads / 32 - 1) / (kEvaluateThreads / 32));
-#endif
     if ((args->affine & kAffinePlain) == kAffinePlain)
       return LaunchVariant(EvaluateKernel<kVariantPlainAll, true, false, Functor, Loss, kRes, Ns...>,
                            kAffineCtas, Computed::kJetBytes, args, s);
@@ -1699,7 +1518,6 @@ int LaunchEvaluate(const cb200_launch_args* args, void* stream) {
     return LaunchVariant(EvaluateKernel<kVariantGenericAll, false, false, Functor, Loss, kRes, Ns...>,
                          kJetCtas, Tables::kJetBytes, args, s);
   }
-#endif
   if (args->plain)
     return LaunchVariant(EvaluateKernel<kVariantPlain, false, false, Functor, Loss, kRes, Ns...>, kJetCtas,
                          Tables::kJetBytes, args, s);
@@ -1723,8 +1541,7 @@ cb200_residual_type MakeResidualType() {
   t.functor_size = static_cast<int32_t>(sizeof(Functor));
   t.loss_size = static_cast<int32_t>(sizeof(Loss));
   t.threads_per_block = kEvaluateThreads;
-  // (the chunked variant is one of the all-outputs specialisations)
-  t.supports_chunks = CB200_KERNEL_CHUNKED_EXCHANGE && CB200_KERNEL_SPECIALISE_ALL_OUTPUTS;
+  t.supports_chunks = 1;
   t.launch = &LaunchEvaluate<Functor, Loss, kRes, Ns...>;
   t.normal_product = &LaunchNormalProduct<kRes, Ns...>;
   return t;

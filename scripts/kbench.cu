@@ -1,7 +1,8 @@
 // Stand-alone micro-benchmark of the BAL evaluation kernel: builds a synthetic
 // BAL-shaped table set directly in C++ (no engine, no Python) and times
-// LaunchEvaluate<SnavelyReprojectionError, HuberLossCUDA, 2, 9, 3>.  Compiled several
-// times with different -DCB200_KERNEL_* settings to A/B kernel variants on the GPU.
+// LaunchEvaluate<SnavelyReprojectionError, HuberLossCUDA, 2, 9, 3>.  To A/B a kernel
+// variant on the GPU, edit evaluate_kernel.cuh in a scratch copy of the tree and build
+// both copies with scripts/kbench_build.sh.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -Iinclude \
 //        -Iceres-solver-cuda_b200/include -Iceres-solver-cuda_b200/examples scripts/kbench.cu
 #include <algorithm>
@@ -108,7 +109,8 @@ int main(int argc, char** argv) {
       jpos[i] = 22 * (int)i + 3; jpos[n + i] = 22 * (int)i;
     }
   }
-  const int grid_max = std::min((n + CB200_EVALUATE_THREADS - 1) / CB200_EVALUATE_THREADS, 4096);
+  constexpr int kThreads = ceres::internal::kEvaluateThreads;
+  const int grid_max = std::min((n + kThreads - 1) / kThreads, 4096);
   a.cost_partial_count = grid_max;
   a.functors = Upload(functors);
   std::vector<char> lb((char*)&loss, (char*)&loss + sizeof(loss));
@@ -203,12 +205,11 @@ int main(int argc, char** argv) {
   }
   {
     using Plan = ceres::internal::SmemPlan<Functor, false, 2, 9, 3>;
-    std::printf("smem plan: %d bytes per CTA, %d CTAs per SM, Jacobian staged %d, stages %d, gather %d, passes %d\n",
-                Plan::kJetBytes, Plan::kCtas, (int)Plan::kStageJacobian, Plan::kStages, CB200_KERNEL_GATHER,
+    std::printf("smem plan: %d bytes per CTA, %d CTAs per SM, Jacobian staged %d, passes %d\n",
+                Plan::kJetBytes, Plan::kCtas, (int)Plan::kStageJacobian,
                 ceres::internal::PassPlan<2, 9, 3>::kNumPasses);
   }
-  std::printf("KBENCH %s ctas=%d affine=%d fma_check=%d stage_g=%d stage_j=%d g=%d j=%d : mean %.3f ms best %.3f ms  (%.2f G blocks/s)  status=%d cost=%.6e\n",
-              argc > 6 ? argv[6] : "", CB200_RESIDENT_CTAS_SMALL, affine, CB200_KERNEL_FMA_CHECK,
-              CB200_KERNEL_STAGE_GRADIENT, CB200_KERNEL_STAGE_JACOBIAN, want_g, want_j, sum / reps, best, n / (sum / reps) / 1e6, st, cost);
+  std::printf("KBENCH %s affine=%d g=%d j=%d : mean %.3f ms best %.3f ms  (%.2f G blocks/s)  status=%d cost=%.6e\n",
+              argc > 6 ? argv[6] : "", affine, want_g, want_j, sum / reps, best, n / (sum / reps) / 1e6, st, cost);
   return 0;
 }
