@@ -26,11 +26,7 @@ class PinnedVector {
   explicit PinnedVector(size_t n = 0, double value = 0.0) { assign(n, value); }
   ~PinnedVector() { Release(); }
   PinnedVector(const PinnedVector&) = delete;
-  PinnedVector& operator=(const PinnedVector& other) {
-    if (size_ != other.size_) assign(other.size_, 0.0);
-    std::copy(other.begin(), other.end(), begin());
-    return *this;
-  }
+  PinnedVector& operator=(const PinnedVector&) = delete;
   void assign(size_t n, double value) {
     if (n != size_) {
       Release();
@@ -42,15 +38,10 @@ class PinnedVector {
     }
     std::fill(begin(), end(), value);
   }
-  size_t size() const { return size_; }
   double* data() { return data_; }
-  const double* data() const { return data_; }
   double& operator[](size_t i) { return data_[i]; }
-  const double& operator[](size_t i) const { return data_[i]; }
   double* begin() { return data_; }
   double* end() { return data_ + size_; }
-  const double* begin() const { return data_; }
-  const double* end() const { return data_ + size_; }
 
  private:
   void Release() {
@@ -60,11 +51,6 @@ class PinnedVector {
   }
   double* data_ = nullptr;
   size_t size_ = 0;
-};
-
-// Wall-clock buckets of the trust-region loop, printed when CB200_SOLVER_TIMING is set.
-struct Buckets {
-  double diagonal = 0, scaling = 0, step = 0, plus = 0, bookkeeping = 0;
 };
 
 // Element-wise pass over [0, n) on num_threads threads; f(i) must only touch index i.
@@ -202,15 +188,225 @@ std::string Solver::Summary::FullReport() const {
   return buf;
 }
 
-// The trust-region loop with state, step, gradient and diagonals resident in HBM
-// (cb200_engine_trust_region_step and friends, include/ceres_b200.h): per iteration the host
-// reads a handful of scalars.  Same decisions as the host loop below
-// (trust_region_minimizer.cc step acceptance, levenberg_marquardt_strategy.cc radius update).
-// Returns false when the program needs the host loop (bounds, a manifold only the host knows,
-// an EvaluationCallback that must see the parameter blocks).
 namespace {
-bool DeviceLoopPossible(const Solver::Options& options, const internal::Program& program,
-                        const internal::ProblemImpl& problem) {
+// The Levenberg-Marquardt loop (trust_region_minimizer.cc step acceptance,
+// levenberg_marquardt_strategy.cc radius update) is written once, in Minimize.  What an
+// iteration asks of the place where the state, gradient and Jacobian live is behind
+// TrustRegionState: DeviceState keeps them in HBM, HostState in host memory.
+// kRejected: an evaluation or the step failed numerically; kError: an engine call failed,
+// and error() holds the call's name and the engine's message.
+enum Result { kDone, kRejected, kError };
+
+// levenberg_marquardt_strategy.cc:97-118: inexact step, stopped by the relative decrease of
+// the quadratic model (eta) and not by the residual (r_tolerance = -1)
+cb200_cgnr_options ConjugateGradientOptions(const Solver::Options& options) {
+  return {options.min_linear_solver_iterations, options.max_linear_solver_iterations, -1.0,
+          options.eta};
+}
+
+class TrustRegionState {
+ public:
+  virtual ~TrustRegionState() = default;
+  // Cost, gradient and Jacobian at the accepted state (the first call: the initial state).
+  virtual Result EvaluateJacobian(double* cost) = 0;
+  // J <- J diag(scale); compute: scale = 1 / (1 + sqrt(diag(J'J))) of this Jacobian first.
+  virtual Result ScaleJacobian(bool compute) = 0;
+  // LM diagonal, linear solve, delta = -y * scale, the norms and the candidate x (+) delta,
+  // reported as the engine's trust-region step reports them.
+  virtual Result ComputeStep(double radius, bool reuse_diagonal, cb200_step_summary* step) = 0;
+  virtual Result EvaluateCandidate(double* cost) = 0;  // cost only
+  virtual void AcceptCandidate() = 0;
+  virtual double GradientMaxNorm() = 0;
+  // The accepted state into the caller's x; evaluation counts, evaluation and linear solver
+  // times into the summary.
+  virtual void Finish(Solver::Summary* summary) = 0;
+  const std::string& error() const { return error_; }
+
+ protected:
+  Result Fail(cb200_engine* engine, const char* call) {
+    error_ = std::string(call) + ": " + cb200_engine_last_error(engine);
+    return kError;
+  }
+  std::string error_;
+};
+
+// State, step, gradient and diagonals in HBM (cb200_engine_trust_region_step and friends,
+// include/ceres_b200.h): per iteration the host reads a handful of scalars.  The state
+// crosses PCIe twice, up and down at the end, and HostState's work vectors are never
+// allocated: page-locking those costs 0.5 s on BAL L.
+class DeviceState final : public TrustRegionState {
+ public:
+  DeviceState(const Solver::Options& options, cb200_engine* engine, double* x)
+      : options_(options), engine_(engine), x_(x) {}
+  Result EvaluateJacobian(double* cost) override {
+    if (!uploaded_ && cb200_engine_state_upload(engine_, x_) != CB200_OK)
+      return Fail("cb200_engine_state_upload");
+    uploaded_ = true;
+    return Evaluate(0, true, cost);
+  }
+  Result ScaleJacobian(bool compute) override {
+    if (cb200_engine_jacobi_scale(engine_, compute) != CB200_OK) return Fail("cb200_engine_jacobi_scale");
+    return kDone;
+  }
+  Result ComputeStep(double radius, bool reuse_diagonal, cb200_step_summary* step) override {
+    cb200_step_options so{};
+    so.radius = radius;
+    so.min_lm_diagonal = options_.min_lm_diagonal;
+    so.max_lm_diagonal = options_.max_lm_diagonal;
+    so.reuse_diagonal = reuse_diagonal;
+    so.cg = ConjugateGradientOptions(options_);
+    const double ls_start = Seconds();
+    if (cb200_engine_trust_region_step(engine_, &so, step) != CB200_OK)
+      return Fail("cb200_engine_trust_region_step");
+    linear_solver_seconds_ += Seconds() - ls_start;
+    return kDone;
+  }
+  Result EvaluateCandidate(double* cost) override { return Evaluate(1, false, cost); }
+  void AcceptCandidate() override { cb200_engine_accept_candidate(engine_); }
+  double GradientMaxNorm() override {
+    double gmax = 0.0;
+    cb200_engine_gradient_max_norm(engine_, &gmax);
+    return gmax;
+  }
+  void Finish(Solver::Summary* summary) override {
+    cb200_engine_state_download(engine_, 0, x_);
+    summary->linear_solver_time_in_seconds = linear_solver_seconds_;
+    summary->residual_evaluation_time_in_seconds = evaluation_seconds_[0];
+    summary->num_residual_evaluations = evaluation_calls_[0];
+    summary->jacobian_evaluation_time_in_seconds = evaluation_seconds_[1];
+    summary->num_jacobian_evaluations = evaluation_calls_[1];
+  }
+
+ private:
+  Result Fail(const char* call) { return TrustRegionState::Fail(engine_, call); }
+  // at state slot `which`: 0 the accepted state, 1 the candidate
+  Result Evaluate(int which, bool jacobian, double* cost) {
+    const double t0 = Seconds();
+    const int rc = cb200_engine_evaluate_state(
+        engine_, which,
+        CB200_APPLY_LOSS_FUNCTION | CB200_KEEP_JACOBIAN_ON_DEVICE | CB200_KEEP_RESIDUALS_ON_DEVICE,
+        jacobian, jacobian, jacobian, cost);
+    evaluation_seconds_[jacobian] += Seconds() - t0;
+    ++evaluation_calls_[jacobian];
+    if (rc < 0) return Fail("cb200_engine_evaluate_state");
+    return rc == CB200_OK ? kDone : kRejected;
+  }
+
+  const Solver::Options& options_;
+  cb200_engine* const engine_;
+  double* const x_;
+  bool uploaded_ = false;
+  double linear_solver_seconds_ = 0.0, evaluation_seconds_[2] = {0.0, 0.0};
+  int evaluation_calls_[2] = {0, 0};
+};
+
+// State, gradient, step and diagonals in host memory around the evaluator.  The linear solve
+// runs where the evaluator keeps the Jacobian: conjugate gradients in HBM for a
+// device-resident one (cb200_engine_cgnr_solve), SolveNormalEquations for a host one.
+class HostState final : public TrustRegionState {
+ public:
+  HostState(const Solver::Options& options, const internal::Program& program,
+            internal::Evaluator* evaluator, internal::SparseMatrix* jacobian, PinnedVector* x)
+      : options_(options), evaluator_(evaluator), jacobian_(jacobian),
+        resident_(dynamic_cast<internal::DeviceResidentJacobian*>(jacobian)),
+        n_(program.NumParameters()), ne_(program.NumEffectiveParameters()),
+        nt_(std::max(1, options.num_threads)), x_(*x), x_plus_(n_), gradient_(ne_),
+        scale_(ne_, 1.0), diagonal_(ne_), D2_(ne_), y_(ne_), delta_(ne_) {
+    // only the host linear solver reads the residuals and the model on the host; with a
+    // device-resident Jacobian the residuals stay on the device as well
+    if (!resident_) {
+      residuals_.resize(program.NumResiduals());
+      model_.resize(program.NumResiduals());
+    }
+  }
+  Result EvaluateJacobian(double* cost) override {
+    double* const residuals = resident_ ? nullptr : residuals_.data();
+    const bool ok = evaluator_->Evaluate(x_.data(), cost, residuals, gradient_.data(), jacobian_);
+    return ok ? kDone : kRejected;
+  }
+  Result ScaleJacobian(bool compute) override {
+    if (compute) {
+      jacobian_->SquaredColumnNorm(scale_.data());
+      ForEach(nt_, ne_, [&](int64_t i) { scale_[i] = 1.0 / (1.0 + std::sqrt(scale_[i])); });
+    }
+    jacobian_->ScaleColumns(scale_.data());
+    return kDone;
+  }
+  Result ComputeStep(double radius, bool reuse_diagonal, cb200_step_summary* step) override {
+    if (!reuse_diagonal) {
+      jacobian_->SquaredColumnNorm(diagonal_.data());
+      ForEach(nt_, ne_, [&](int64_t i) {
+        diagonal_[i] =
+            std::min(std::max(diagonal_[i], options_.min_lm_diagonal), options_.max_lm_diagonal);
+      });
+    }
+    ForEach(nt_, ne_, [&](int64_t i) { D2_[i] = diagonal_[i] / radius; });
+    const double ls_start = Seconds();
+    if (resident_) {
+      const cb200_cgnr_options cg_options = ConjugateGradientOptions(options_);
+      y_.assign(ne_, 0.0);
+      if (cb200_engine_cgnr_solve(resident_->engine(), D2_.data(), &cg_options, y_.data(),
+                                  &step->cg) != CB200_OK)
+        return Fail(resident_->engine(), "cb200_engine_cgnr_solve");
+      // step = -y: model cost change = (J y).r - |J y|^2 / 2
+      step->model_cost_change = step->cg.jy_dot_b - 0.5 * step->cg.jy_squared_norm;
+      ForEach(nt_, ne_, [&](int64_t i) { y_[i] = -y_[i]; });
+    } else {
+      step->cg.num_iterations =
+          SolveNormalEquations(*jacobian_, D2_.data(), residuals_.data(),
+                               options_.max_linear_solver_iterations, 1e-2 * options_.eta, &y_);
+      // step = -y (scaled space); model cost change = -m'(r + m/2), m = J step
+      std::fill(model_.begin(), model_.end(), 0.0);
+      for (int i = 0; i < ne_; ++i) y_[i] = -y_[i];
+      jacobian_->RightMultiplyAndAccumulate(y_.data(), model_.data());
+      double model_cost_change = 0.0;
+      for (size_t i = 0; i < model_.size(); ++i)
+        model_cost_change -= model_[i] * (residuals_[i] + 0.5 * model_[i]);
+      step->model_cost_change = model_cost_change;
+    }
+    linear_solver_seconds_ += Seconds() - ls_start;
+    ForEach(nt_, ne_, [&](int64_t i) { delta_[i] = y_[i] * scale_[i]; });
+    step->step_norm = std::sqrt(Reduce(nt_, ne_, false, [&](int64_t i) { return delta_[i] * delta_[i]; }));
+    step->state_norm = std::sqrt(Reduce(nt_, n_, false, [&](int64_t i) { return x_[i] * x_[i]; }));
+    step->plus_ok = step->cg.termination != 2 && step->model_cost_change > 0.0 &&
+                    evaluator_->Plus(x_.data(), delta_.data(), x_plus_.data());
+    return kDone;
+  }
+  Result EvaluateCandidate(double* cost) override {
+    return evaluator_->Evaluate(x_plus_.data(), cost, nullptr, nullptr, nullptr) ? kDone : kRejected;
+  }
+  void AcceptCandidate() override { ForEach(nt_, n_, [&](int64_t i) { x_[i] = x_plus_[i]; }); }
+  double GradientMaxNorm() override {
+    return Reduce(nt_, ne_, true, [&](int64_t i) { return std::fabs(gradient_[i]); });
+  }
+  void Finish(Solver::Summary* summary) override {
+    summary->linear_solver_time_in_seconds = linear_solver_seconds_;
+    for (const auto& kv : evaluator_->Statistics()) {
+      if (kv.first == "Evaluator::Residual") {
+        summary->residual_evaluation_time_in_seconds = kv.second.time;
+        summary->num_residual_evaluations = kv.second.calls;
+      } else if (kv.first == "Evaluator::Jacobian") {
+        summary->jacobian_evaluation_time_in_seconds = kv.second.time;
+        summary->num_jacobian_evaluations = kv.second.calls;
+      }
+    }
+  }
+
+ private:
+  const Solver::Options& options_;
+  internal::Evaluator* const evaluator_;
+  internal::SparseMatrix* const jacobian_;
+  internal::DeviceResidentJacobian* const resident_;
+  const int n_, ne_, nt_;
+  double linear_solver_seconds_ = 0.0;
+  PinnedVector& x_;
+  PinnedVector x_plus_, gradient_, scale_, diagonal_, D2_, y_;
+  std::vector<double> delta_, residuals_, model_;
+};
+
+// The state stays in HBM unless the program needs the host: bounds, a manifold only the host
+// knows, an EvaluationCallback that must see the parameter blocks.
+bool DeviceLoopPossible(const internal::Program& program, const internal::ProblemImpl& problem) {
   if (std::getenv("CB200_HOST_TRUST_REGION")) return false;
   if (problem.options().evaluation_callback != nullptr) return false;
   for (const internal::ParameterBlock* pb : program.parameter_blocks()) {
@@ -221,35 +417,22 @@ bool DeviceLoopPossible(const Solver::Options& options, const internal::Program&
   return true;
 }
 
-void MinimizeOnDevice(const Solver::Options& options, cb200_engine* engine, double fixed_cost,
-                      double start, double* x, Solver::Summary* summary) {
-  auto fail = [&](const char* what) {
+// Returns without Finish when the initial evaluation or Jacobi scaling fails.
+void Minimize(const Solver::Options& options, TrustRegionState* state, double fixed_cost,
+              double start, Solver::Summary* summary) {
+  auto fail = [&](const std::string& message) {
     summary->termination_type = FAILURE;
-    summary->message = std::string(what) + ": " + cb200_engine_last_error(engine);
-  };
-  const uint32_t kLoss = CB200_APPLY_LOSS_FUNCTION;
-  double evaluation_seconds[2] = {0.0, 0.0};
-  int evaluation_calls[2] = {0, 0};
-  auto evaluate = [&](int which, bool jacobian, double* cost) {
-    const double t0 = Seconds();
-    const int rc = cb200_engine_evaluate_state(
-        engine, which, kLoss | CB200_KEEP_JACOBIAN_ON_DEVICE | CB200_KEEP_RESIDUALS_ON_DEVICE,
-        jacobian, jacobian, jacobian, cost);
-    evaluation_seconds[jacobian] += Seconds() - t0;
-    ++evaluation_calls[jacobian];
-    return rc;
+    summary->message = message;
   };
   double cost = 0.0;
-  if (cb200_engine_state_upload(engine, x) != CB200_OK) return fail("cb200_engine_state_upload");
-  int rc = evaluate(0, true, &cost);
-  if (rc != CB200_OK) {
+  Result result = state->EvaluateJacobian(&cost);
+  if (result != kDone) {
     summary->message = "Initial residual and Jacobian evaluation failed.";
-    if (rc < 0) fail("cb200_engine_evaluate_state");
+    if (result == kError) fail(state->error());
     return;
   }
   summary->initial_cost = cost + fixed_cost;
-  if (options.jacobi_scaling && cb200_engine_jacobi_scale(engine, 1) != CB200_OK)
-    return fail("cb200_engine_jacobi_scale");
+  if (options.jacobi_scaling && state->ScaleJacobian(true) != kDone) return fail(state->error());
   double radius = options.initial_trust_region_radius, decrease_factor = 2.0;
   bool reuse_diagonal = false;
   summary->termination_type = NO_CONVERGENCE;
@@ -258,58 +441,38 @@ void MinimizeOnDevice(const Solver::Options& options, cb200_engine* engine, doub
     std::printf("iter      cost      cost_change  |gradient|   |step|    tr_ratio  tr_radius  ls_iter\n"
                 "%4d  %.6e    %.2e   %.2e   %.2e  %.2e  %.2e   %5d\n",
                 0, cost + fixed_cost, 0.0, 0.0, 0.0, 0.0, radius, 0);
+  const bool timing = std::getenv("CB200_SOLVER_TIMING") != nullptr;
   for (int it = 1; it <= options.max_num_iterations; ++it) {
     if (Seconds() - start > options.max_solver_time_in_seconds) {
       summary->message = "Maximum solver time reached.";
       break;
     }
-    cb200_step_options so{};
-    so.radius = radius;
-    so.min_lm_diagonal = options.min_lm_diagonal;
-    so.max_lm_diagonal = options.max_lm_diagonal;
-    so.reuse_diagonal = reuse_diagonal;
-    so.cg.min_num_iterations = options.min_linear_solver_iterations;
-    so.cg.max_num_iterations = options.max_linear_solver_iterations;
-    so.cg.r_tolerance = -1.0;
-    so.cg.q_tolerance = options.eta;  // levenberg_marquardt_strategy.cc:97-118
-    cb200_step_summary ss;
-    const double ls_start = Seconds();
-    if (cb200_engine_trust_region_step(engine, &so, &ss) != CB200_OK) {
-      fail("cb200_engine_trust_region_step");
-      break;
-    }
-    summary->linear_solver_time_in_seconds += Seconds() - ls_start;
-    if (std::getenv("CB200_SOLVER_TIMING"))
-      std::fprintf(stderr, "iteration %d: trust-region step %.1f ms wall, conjugate gradients %.1f ms "
-                   "on the device (%d iterations)\n", it, (Seconds() - ls_start) * 1e3,
-                   ss.cg.solve_ms, ss.cg.num_iterations);
+    cb200_step_summary step{};
+    const double step_start = Seconds();
+    if (state->ComputeStep(radius, reuse_diagonal, &step) != kDone) { fail(state->error()); break; }
+    if (timing)
+      std::fprintf(stderr, "iteration %d: trust-region step %.1f ms wall, %d linear solver iterations, "
+                   "%.1f ms of them on the device\n", it, (Seconds() - step_start) * 1e3,
+                   step.cg.num_iterations, step.cg.solve_ms);
     Solver::IterationSummary is;
     is.iteration = it;
-    is.linear_solver_iterations = ss.cg.num_iterations;
-    is.step_norm = ss.step_norm;
+    is.linear_solver_iterations = step.cg.num_iterations;
+    is.step_norm = step.step_norm;
     double new_cost = 0.0;
-    bool ok = ss.cg.termination != 2 && ss.model_cost_change > 0.0 && ss.plus_ok;
+    bool ok = step.cg.termination != 2 && step.model_cost_change > 0.0 && step.plus_ok;
     if (ok) {
-      rc = evaluate(1, false, &new_cost);
-      if (rc < 0) { fail("cb200_engine_evaluate_state"); break; }
-      ok = rc == CB200_OK;
+      result = state->EvaluateCandidate(&new_cost);
+      if (result == kError) { fail(state->error()); break; }
+      ok = result == kDone;
     }
-    const double relative_decrease = ok ? (cost - new_cost) / ss.model_cost_change : -1.0;
+    const double relative_decrease = ok ? (cost - new_cost) / step.model_cost_change : -1.0;
     is.relative_decrease = relative_decrease;
     if (ok && relative_decrease > options.min_relative_decrease) {
       is.step_is_successful = true;
       is.cost_change = cost - new_cost;
-      cb200_engine_accept_candidate(engine);
-      rc = evaluate(0, true, &cost);
-      if (rc != CB200_OK) {
-        summary->termination_type = FAILURE;
-        summary->message = "Residual and Jacobian evaluation failed.";
-        break;
-      }
-      if (options.jacobi_scaling && cb200_engine_jacobi_scale(engine, 0) != CB200_OK) {
-        fail("cb200_engine_jacobi_scale");
-        break;
-      }
+      state->AcceptCandidate();
+      if (state->EvaluateJacobian(&cost) != kDone) { fail("Residual and Jacobian evaluation failed."); break; }
+      if (options.jacobi_scaling && state->ScaleJacobian(false) != kDone) { fail(state->error()); break; }
       radius = std::min(options.max_trust_region_radius,
                         radius / std::max(1.0 / 3.0, 1.0 - std::pow(2.0 * relative_decrease - 1.0, 3)));
       decrease_factor = 2.0;
@@ -321,43 +484,31 @@ void MinimizeOnDevice(const Solver::Options& options, cb200_engine* engine, doub
       reuse_diagonal = true;
       ++summary->num_unsuccessful_steps;
     }
-    double gmax = 0.0;
-    cb200_engine_gradient_max_norm(engine, &gmax);
+    const double gmax = state->GradientMaxNorm();
     is.cost = cost + fixed_cost;
     is.gradient_max_norm = gmax;
     is.trust_region_radius = radius;
     summary->iterations.push_back(is);
     if (options.minimizer_progress_to_stdout)
       std::printf("%4d  %.6e    %.2e   %.2e   %.2e  %.2e  %.2e   %5d\n", it, is.cost, is.cost_change,
-                  gmax, ss.step_norm, relative_decrease, radius, ss.cg.num_iterations);
-    if (is.step_is_successful) {
-      if (std::fabs(is.cost_change) <= options.function_tolerance * cost) {
-        summary->termination_type = CONVERGENCE;
-        summary->message = "Function tolerance reached.";
-        break;
-      }
-      if (gmax <= options.gradient_tolerance) {
-        summary->termination_type = CONVERGENCE;
-        summary->message = "Gradient tolerance reached.";
-        break;
-      }
-      if (ss.step_norm <= options.parameter_tolerance * (ss.state_norm + options.parameter_tolerance)) {
-        summary->termination_type = CONVERGENCE;
-        summary->message = "Parameter tolerance reached.";
-        break;
-      }
-    } else if (radius < options.min_trust_region_radius) {
+                  gmax, step.step_norm, relative_decrease, radius, step.cg.num_iterations);
+    const char* converged = nullptr;
+    if (!is.step_is_successful)
+      converged = radius < options.min_trust_region_radius ? "Minimum trust region radius reached." : nullptr;
+    else if (std::fabs(is.cost_change) <= options.function_tolerance * cost)
+      converged = "Function tolerance reached.";
+    else if (gmax <= options.gradient_tolerance)
+      converged = "Gradient tolerance reached.";
+    else if (step.step_norm <= options.parameter_tolerance * (step.state_norm + options.parameter_tolerance))
+      converged = "Parameter tolerance reached.";
+    if (converged) {
       summary->termination_type = CONVERGENCE;
-      summary->message = "Minimum trust region radius reached.";
+      summary->message = converged;
       break;
     }
   }
-  cb200_engine_state_download(engine, 0, x);
+  state->Finish(summary);
   summary->final_cost = cost + fixed_cost;
-  summary->residual_evaluation_time_in_seconds = evaluation_seconds[0];
-  summary->num_residual_evaluations = evaluation_calls[0];
-  summary->jacobian_evaluation_time_in_seconds = evaluation_seconds[1];
-  summary->num_jacobian_evaluations = evaluation_calls[1];
 }
 }  // namespace
 
@@ -484,201 +635,17 @@ void Solver::Solve(const Options& options, Problem* problem, Summary* summary) {
 
   // ---- trust-region loop
   const double minimizer_start = Seconds();
-  const int n = program->NumParameters(), ne = program->NumEffectiveParameters();
-  const int m = program->NumResiduals();
-  const int nt = std::max(1, options.num_threads);
-  Buckets buckets;
-  PinnedVector x(n);
+  PinnedVector x(program->NumParameters());
   program->ParameterBlocksToStateVector(x.data());
   auto* resident = dynamic_cast<internal::DeviceResidentJacobian*>(jacobian.get());
-  if (resident && DeviceLoopPossible(options, *program, *impl)) {
-    // (the loop on the device needs the state on the host twice - up, and down at the end -
-    // and none of the host loop's work vectors: page-locking those cost 0.5 s on BAL L)
-    MinimizeOnDevice(options, resident->engine(), fixed_cost, start, x.data(), summary);
-    program->StateVectorToParameterBlocks(x.data());  // results back into the user's arrays
-    summary->minimizer_time_in_seconds = Seconds() - minimizer_start;
-    summary->total_time_in_seconds = Seconds() - start;
-    return;
-  }
-  PinnedVector x_plus(n), gradient(ne), scale(ne, 1.0), diagonal(ne), D2(ne), y(ne);
-  std::vector<double> delta(ne);
-  // only the host linear solver reads the residuals and the model on the host
-  std::vector<double> residuals, model;
-  // with a device-resident Jacobian the residuals stay on the device as well
-  if (!resident) {
-    residuals.resize(m);
-    model.resize(m);
-  }
-  double* const residuals_out = resident ? nullptr : residuals.data();
-  double cost = 0.0;
-  if (!evaluator->Evaluate(x.data(), &cost, residuals_out, gradient.data(), jacobian.get())) {
-    summary->message = "Initial residual and Jacobian evaluation failed.";
-    return;
-  }
-  summary->initial_cost = cost + fixed_cost;
-  if (options.jacobi_scaling) {
-    jacobian->SquaredColumnNorm(scale.data());
-    ForEach(nt, ne, [&](int64_t i) { scale[i] = 1.0 / (1.0 + std::sqrt(scale[i])); });
-    jacobian->ScaleColumns(scale.data());
-  }
-  double radius = options.initial_trust_region_radius, decrease_factor = 2.0;
-  bool reuse_diagonal = false;
-  summary->termination_type = NO_CONVERGENCE;
-  summary->message = "Maximum number of iterations reached.";
-  if (options.minimizer_progress_to_stdout)
-    std::printf("iter      cost      cost_change  |gradient|   |step|    tr_ratio  tr_radius  ls_iter\n"
-                "%4d  %.6e    %.2e   %.2e   %.2e  %.2e  %.2e   %5d\n",
-                0, cost + fixed_cost, 0.0, 0.0, 0.0, 0.0, radius, 0);
-  for (int it = 1; it <= options.max_num_iterations; ++it) {
-    if (Seconds() - start > options.max_solver_time_in_seconds) {
-      summary->message = "Maximum solver time reached.";
-      break;
-    }
-    double mark = Seconds();
-    auto lap = [&](double* bucket) {
-      const double now = Seconds();
-      *bucket += now - mark;
-      mark = now;
-    };
-    if (!reuse_diagonal) {
-      jacobian->SquaredColumnNorm(diagonal.data());
-      ForEach(nt, ne, [&](int64_t i) {
-        diagonal[i] =
-            std::min(std::max(diagonal[i], options.min_lm_diagonal), options.max_lm_diagonal);
-      });
-    }
-    ForEach(nt, ne, [&](int64_t i) { D2[i] = diagonal[i] / radius; });
-    lap(&buckets.diagonal);
-    const double ls_start = Seconds();
-    int ls_iterations = 0;
-    double model_cost_change = 0.0, step_norm = 0.0, x_norm = 0.0;
-    bool linear_solver_ok = true;
-    if (resident) {
-      // levenberg_marquardt_strategy.cc:97-118: inexact step, stopped by the relative
-      // decrease of the quadratic model (eta)
-      cb200_cgnr_options cg_options;
-      cg_options.min_num_iterations = options.min_linear_solver_iterations;
-      cg_options.max_num_iterations = options.max_linear_solver_iterations;
-      cg_options.r_tolerance = -1.0;
-      cg_options.q_tolerance = options.eta;
-      cb200_cgnr_summary cg;
-      y.assign(ne, 0.0);
-      if (cb200_engine_cgnr_solve(resident->engine(), D2.data(), &cg_options, y.data(), &cg) !=
-          CB200_OK) {
-        summary->termination_type = FAILURE;
-        summary->message = std::string("cb200_engine_cgnr_solve: ") +
-                           cb200_engine_last_error(resident->engine());
-        break;
-      }
-      ls_iterations = cg.num_iterations;
-      linear_solver_ok = cg.termination != 2;
-      // step = -y: model cost change = (J y).r - |J y|^2 / 2
-      model_cost_change = cg.jy_dot_b - 0.5 * cg.jy_squared_norm;
-      ForEach(nt, ne, [&](int64_t i) { y[i] = -y[i]; });
-    } else {
-      ls_iterations = SolveNormalEquations(*jacobian, D2.data(), residuals.data(),
-                                           options.max_linear_solver_iterations,
-                                           1e-2 * options.eta, &y);
-      // step = -y (scaled space); model cost change = -m'(r + m/2), m = J step
-      std::fill(model.begin(), model.end(), 0.0);
-      for (int i = 0; i < ne; ++i) y[i] = -y[i];
-      jacobian->RightMultiplyAndAccumulate(y.data(), model.data());
-      for (int i = 0; i < m; ++i) model_cost_change -= model[i] * (residuals[i] + 0.5 * model[i]);
-    }
-    summary->linear_solver_time_in_seconds += Seconds() - ls_start;
-    mark = Seconds();
-    ForEach(nt, ne, [&](int64_t i) { delta[i] = y[i] * scale[i]; });
-    step_norm = Reduce(nt, ne, false, [&](int64_t i) { return delta[i] * delta[i]; });
-    x_norm = Reduce(nt, n, false, [&](int64_t i) { return x[i] * x[i]; });
-    step_norm = std::sqrt(step_norm);
-    IterationSummary is;
-    is.iteration = it;
-    is.linear_solver_iterations = ls_iterations;
-    is.step_norm = step_norm;
-    double new_cost = 0.0;
-    lap(&buckets.step);
-    bool ok = linear_solver_ok && model_cost_change > 0.0 &&
-              evaluator->Plus(x.data(), delta.data(), x_plus.data());
-    lap(&buckets.plus);
-    ok = ok && evaluator->Evaluate(x_plus.data(), &new_cost, nullptr, nullptr, nullptr);
-    mark = Seconds();
-    const double relative_decrease = ok ? (cost - new_cost) / model_cost_change : -1.0;
-    is.relative_decrease = relative_decrease;
-    if (ok && relative_decrease > options.min_relative_decrease) {
-      is.step_is_successful = true;
-      is.cost_change = cost - new_cost;
-      ForEach(nt, n, [&](int64_t i) { x[i] = x_plus[i]; });
-      if (!evaluator->Evaluate(x.data(), &cost, residuals_out, gradient.data(),
-                               jacobian.get())) {
-        summary->termination_type = FAILURE;
-        summary->message = "Residual and Jacobian evaluation failed.";
-        break;
-      }
-      mark = Seconds();
-      if (options.jacobi_scaling) jacobian->ScaleColumns(scale.data());
-      lap(&buckets.scaling);
-      radius = std::min(options.max_trust_region_radius,
-                        radius / std::max(1.0 / 3.0, 1.0 - std::pow(2.0 * relative_decrease - 1.0, 3)));
-      decrease_factor = 2.0;
-      reuse_diagonal = false;
-      ++summary->num_successful_steps;
-    } else {
-      radius /= decrease_factor;
-      decrease_factor *= 2.0;
-      reuse_diagonal = true;
-      ++summary->num_unsuccessful_steps;
-    }
-    mark = Seconds();
-    const double gmax =
-        Reduce(nt, ne, true, [&](int64_t i) { return std::fabs(gradient[i]); });
-    lap(&buckets.bookkeeping);
-    is.cost = cost + fixed_cost;
-    is.gradient_max_norm = gmax;
-    is.trust_region_radius = radius;
-    summary->iterations.push_back(is);
-    if (options.minimizer_progress_to_stdout)
-      std::printf("%4d  %.6e    %.2e   %.2e   %.2e  %.2e  %.2e   %5d\n", it, is.cost, is.cost_change,
-                  gmax, step_norm, relative_decrease, radius, ls_iterations);
-    if (is.step_is_successful) {
-      if (std::fabs(is.cost_change) <= options.function_tolerance * cost) {
-        summary->termination_type = CONVERGENCE;
-        summary->message = "Function tolerance reached.";
-        break;
-      }
-      if (gmax <= options.gradient_tolerance) {
-        summary->termination_type = CONVERGENCE;
-        summary->message = "Gradient tolerance reached.";
-        break;
-      }
-      if (step_norm <= options.parameter_tolerance * (std::sqrt(x_norm) + options.parameter_tolerance)) {
-        summary->termination_type = CONVERGENCE;
-        summary->message = "Parameter tolerance reached.";
-        break;
-      }
-    } else if (radius < options.min_trust_region_radius) {
-      summary->termination_type = CONVERGENCE;
-      summary->message = "Minimum trust region radius reached.";
-      break;
-    }
-  }
+  std::unique_ptr<TrustRegionState> state;
+  if (resident && DeviceLoopPossible(*program, *impl))
+    state.reset(new DeviceState(options, resident->engine(), x.data()));
+  else
+    state.reset(new HostState(options, *program, evaluator.get(), jacobian.get(), &x));
+  Minimize(options, state.get(), fixed_cost, start, summary);
   program->StateVectorToParameterBlocks(x.data());  // results back into the user's arrays
-  summary->final_cost = cost + fixed_cost;
-  for (const auto& kv : evaluator->Statistics()) {
-    if (kv.first == "Evaluator::Residual") {
-      summary->residual_evaluation_time_in_seconds = kv.second.time;
-      summary->num_residual_evaluations = kv.second.calls;
-    } else if (kv.first == "Evaluator::Jacobian") {
-      summary->jacobian_evaluation_time_in_seconds = kv.second.time;
-      summary->num_jacobian_evaluations = kv.second.calls;
-    }
-  }
   summary->minimizer_time_in_seconds = Seconds() - minimizer_start;
-  if (std::getenv("CB200_SOLVER_TIMING"))
-    std::fprintf(stderr,
-                 "solver buckets (s): LM diagonal %.3f, Jacobi scaling %.3f, step vectors %.3f, "
-                 "Plus %.3f, gradient norm %.3f\n",
-                 buckets.diagonal, buckets.scaling, buckets.step, buckets.plus,
-                 buckets.bookkeeping);
   summary->total_time_in_seconds = Seconds() - start;
 }
 
