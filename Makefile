@@ -13,7 +13,7 @@ CXXFLAGS := -O2 -std=c++17 -fPIC -Wall -Wno-unknown-pragmas $(INC) -I/usr/local/
 LIB := $(PKG)/lib/libceres_b200.so
 DRV := tests/driver/libceres_b200_driver.so
 HDRS := $(wildcard include/*.h $(PKG)/include/ceres/*.h $(PKG)/include/ceres/internal/*.h $(PKG)/include/ceres/internal/*.cuh)
-DRV_SRCS := driver_api driver_bal driver_bal2 driver_pose driver_pose3d driver_tests
+DRV_SRCS := driver_api driver_bal driver_bal2 driver_pose driver_pose3d driver_tests driver_preconditioner
 DRV_OBJS := $(patsubst %,build/driver/%.o,$(DRV_SRCS))
 
 EXAMPLE := build/examples/bundle_adjuster

@@ -116,7 +116,8 @@ def driver():
         L.drv_plus.argtypes = [C.c_void_p] * 4
         L.drv_plus_threads.argtypes = [C.c_void_p] * 4 + [C.c_int]
         L.drv_dense_jacobian.argtypes = [C.c_void_p, C.c_void_p]
-        L.drv_solve.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p]
+        L.drv_solve_preconditioned.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                               C.c_void_p, C.c_int, C.c_void_p]
         L.drv_problem_evaluate.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int,
                                            C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         L.drv_problem_evaluate_get.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
@@ -125,10 +126,12 @@ def driver():
         L.drv_jacobian_multiply.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         L.drv_jacobian_squared_column_norm.argtypes = [C.c_void_p, C.c_void_p]
         L.drv_jacobian_scale_columns.argtypes = [C.c_void_p, C.c_void_p]
-        L.drv_cgnr_solve.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_double,
-                                     C.c_double, C.c_void_p, C.c_void_p]
+        L.drv_cgnr_solve_preconditioned.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                                    C.c_double, C.c_double, C.c_int, C.c_void_p,
+                                                    C.c_void_p]
         L.drv_user_values.argtypes = [C.c_void_p, C.c_void_p]
-        L.drv_options_is_valid.argtypes = [C.c_void_p, C.c_int, C.c_char_p, C.c_int]
+        L.drv_options_is_valid_for.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                               C.c_char_p, C.c_int]
         L.drv_argument_slot_ordering.argtypes = [C.c_void_p, C.c_void_p]
         _DRV = L
     return _DRV
@@ -158,12 +161,22 @@ _INT_ARRAYS = {
 # ceres::LinearSolverType values (include/ceres/types.h of this repository)
 SPARSE_NORMAL_CHOLESKY, DENSE_SCHUR, SPARSE_SCHUR, ITERATIVE_SCHUR, CGNR = 2, 3, 4, 5, 6
 
+# Preconditioners by name: (ceres::PreconditionerType, CB200_PRECONDITIONER_*)
+PRECONDITIONERS = {"identity": (0, 2), "jacobi": (1, 1), "scalar_jacobi": (2, 0)}
+
+
+def _preconditioner(name, which):
+    if name not in PRECONDITIONERS:
+        raise ValueError(f"unknown preconditioner {name!r}; one of {sorted(PRECONDITIONERS)}")
+    return PRECONDITIONERS[name][which]
+
 
 def solve(spec, linear_solver_type=ITERATIVE_SCHUR, max_num_iterations=20, ordering=None,
-          device=0, bulk=False, cuda_sparse=False):
+          device=0, bulk=False, cuda_sparse=False, preconditioner="scalar_jacobi"):
     """ceres::Solve(options, ProblemCUDA*, summary) (reference: problem_cuda.h:490-502) on
     a ProblemSpec built through the per-block C++ API.  Returns a dict with the summary
-    and the solution in the specification's parameter-block order."""
+    and the solution in the specification's parameter-block order.  preconditioner: a key of
+    PRECONDITIONERS (Solver::Options::preconditioner_type)."""
     L = driver()
     h = L.drv_create(
         spec.num_pb, _p(spec.pb_size), _p(spec.pb_values), _p(spec.pb_constant),
@@ -173,10 +186,11 @@ def solve(spec, linear_solver_type=ITERATIVE_SCHUR, max_num_iterations=20, order
     err = L.drv_error(h)
     if err:
         raise RuntimeError(err.decode())
-    out = np.zeros(8)
+    out = np.zeros(9)
     o = None if ordering is None else np.ascontiguousarray(ordering, dtype=np.int32)
-    ok = L.drv_solve(h, int(linear_solver_type), int(cuda_sparse), int(max_num_iterations), _p(o),
-                     int(device), _p(out))
+    ok = L.drv_solve_preconditioned(h, int(linear_solver_type), int(cuda_sparse),
+                                    _preconditioner(preconditioner, 0), int(max_num_iterations),
+                                    _p(o), int(device), _p(out))
     x = np.zeros(spec.pb_values.size)
     L.drv_user_values(h, _p(x))
     msg = L.drv_error(h).decode()
@@ -184,7 +198,8 @@ def solve(spec, linear_solver_type=ITERATIVE_SCHUR, max_num_iterations=20, order
     return dict(usable=bool(ok), initial_cost=out[0], final_cost=out[1], iterations=int(out[2]),
                 successful_steps=int(out[3]), termination_type=int(out[4]),
                 jacobian_evaluations=int(out[5]), residual_evaluations=int(out[6]),
-                linear_solver_seconds=float(out[7]), message=msg,
+                linear_solver_seconds=float(out[7]), linear_solver_iterations=int(out[8]),
+                message=msg,
                 x=x)
 
 
@@ -206,9 +221,10 @@ def argument_slot_ordering(spec):
     return bool(found), groups
 
 
-def options_is_valid(spec, minimizer_type):
-    """Solver::Options::IsValid with use_cuda_for_evaluator (reference solver.cc:702-708).
-    Returns (valid, message)."""
+def options_is_valid(spec, minimizer_type, linear_solver_type=None, cuda_sparse=False,
+                     preconditioner=None):
+    """Solver::Options::IsValid with use_cuda_for_evaluator (reference solver.cc:702-708);
+    None keeps an option's default.  Returns (valid, message)."""
     L = driver()
     h = L.drv_create(
         spec.num_pb, _p(spec.pb_size), _p(spec.pb_values), _p(spec.pb_constant),
@@ -216,7 +232,10 @@ def options_is_valid(spec, minimizer_type):
         _p(spec.rb_type), _p(spec.rb_pb), _p(spec.rb_loss_kind), _p(spec.rb_loss_a),
         _p(spec.rb_loss_b), _p(spec.fdata), 0)
     msg = C.create_string_buffer(512)
-    ok = L.drv_options_is_valid(h, int(minimizer_type), msg, 512)
+    ok = L.drv_options_is_valid_for(
+        h, int(minimizer_type), -1 if linear_solver_type is None else int(linear_solver_type),
+        int(cuda_sparse), -1 if preconditioner is None else _preconditioner(preconditioner, 0),
+        msg, 512)
     L.drv_destroy(h)
     return bool(ok), msg.value.decode()
 
@@ -422,14 +441,15 @@ class CudaProblem:
         self._la_check(driver().drv_jacobian_scale_columns(self.h, _p(scale)))
 
     def cgnr_solve(self, d_squared=None, min_iterations=0, max_iterations=500, r_tolerance=-1.0,
-                   q_tolerance=0.1):
-        """(J'J + diag(d_squared)) y = J'r on the device; returns (y, summary dict)."""
+                   q_tolerance=0.1, preconditioner="scalar_jacobi"):
+        """(J'J + diag(d_squared)) y = J'r on the device; returns (y, summary dict).
+        preconditioner: a key of PRECONDITIONERS."""
         d2 = None if d_squared is None else np.ascontiguousarray(d_squared, dtype=np.float64)
         y = np.zeros(self.num_effective_parameters)
         out = np.zeros(8)
-        self._la_check(driver().drv_cgnr_solve(self.h, _p(d2), int(min_iterations),
-                                               int(max_iterations), float(r_tolerance),
-                                               float(q_tolerance), _p(y), _p(out)))
+        self._la_check(driver().drv_cgnr_solve_preconditioned(
+            self.h, _p(d2), int(min_iterations), int(max_iterations), float(r_tolerance),
+            float(q_tolerance), _preconditioner(preconditioner, 1), _p(y), _p(out)))
         return y, dict(iterations=int(out[0]), termination=int(out[1]), gradient_norm=out[2],
                        residual_norm=out[3], jy_dot_b=out[4], jy_squared_norm=out[5], ms=out[6])
 

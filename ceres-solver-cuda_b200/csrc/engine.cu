@@ -292,6 +292,7 @@ struct JacobianWalk {
   const int32_t* jstride;  // [n]
   const int32_t* respos;   // [n]
   const int32_t* pb_table;
+  const int32_t* block_offset;  // kOpBlockDiagonal: cb200_engine::bj_offset
   double* values;
 };
 
@@ -300,14 +301,23 @@ __device__ __forceinline__ void RedAddF64(double* address, double value) {
 }
 
 enum { kOpRight = 0, kOpLeft = 1, kOpColumnNorm = 2, kOpScale = 3, kOpNormal = 4,
-       kOpScaleNorm = 5 };  // kOpScaleNorm: kOpScale with x, then kOpColumnNorm into y (one pass
+       kOpScaleNorm = 5,    // kOpScaleNorm: kOpScale with x, then kOpColumnNorm into y (one pass
                             // in the per-type kernel, two table walks otherwise)
+       kOpBlockDiagonal = 6 };
+
+// Position of entry (a, c), a <= c, of a t x t block stored as its packed upper triangle, row
+// by row.
+__device__ __forceinline__ int PackedUpper(int a, int c, int t) {
+  return a * t - a * (a - 1) / 2 + (c - a);
+}
 
 // One thread per residual block.  x / y meaning per operation:
 //   kOpRight:      y[rows] = sum_c J(r, c) x[c]        (y indexed by local residual)
 //   kOpLeft:       y[c]   += sum_r J(r, c) x[r]        (atomic; x indexed by local residual)
 //   kOpColumnNorm: y[c]   += sum_r J(r, c)^2           (atomic)
 //   kOpScale:      J(r, c) *= x[c]
+//   kOpBlockDiagonal: the upper triangle of C'C of every cell C is added (atomic) to the block
+//                  of its parameter block at y + block_offset[first column]
 template <int kOp>
 __global__ void __launch_bounds__(256) JacobianWalkKernel(const JacobianWalk w,
                                                           const double* __restrict__ x,
@@ -364,33 +374,49 @@ __global__ void __launch_bounds__(256) JacobianWalkKernel(const JacobianWalk w,
         const int tan = w.plain ? w.sizes[j] : w.pb_table[8 * w.pb[at] + 2];
         const int rs = w.crs ? w.jstride[i] : tan;
         double* v = w.values + jp;
-        for (int c0 = 0; c0 < tan; c0 += kChunk) {
-          if (kOp == kOpScale) {
-            double sc[kChunk];
+        if constexpr (kOp == kOpBlockDiagonal) {
+          // the cell is read tan * (tan + 1) / 2 times; after the first pass from L1
+          double* out = y + w.block_offset[col];
+          int k = 0;
+          for (int a = 0; a < tan; ++a) {
+            for (int c = a; c < tan; ++c, ++k) {
+              double acc = 0.0;
+              for (int r = 0; r < w.kres; ++r) {
+                const double* row = v + static_cast<size_t>(r) * rs;
+                acc = fma(row[a], row[c], acc);
+              }
+              RedAddF64(out + k, acc);
+            }
+          }
+        } else {
+          for (int c0 = 0; c0 < tan; c0 += kChunk) {
+            if (kOp == kOpScale) {
+              double sc[kChunk];
 #pragma unroll
-            for (int k = 0; k < kChunk; ++k) sc[k] = c0 + k < tan ? x[col + c0 + k] : 1.0;
-            for (int r = 0; r < w.kres; ++r) {
-              double* row = v + static_cast<size_t>(r) * rs + c0;
+              for (int k = 0; k < kChunk; ++k) sc[k] = c0 + k < tan ? x[col + c0 + k] : 1.0;
+              for (int r = 0; r < w.kres; ++r) {
+                double* row = v + static_cast<size_t>(r) * rs + c0;
+#pragma unroll
+                for (int k = 0; k < kChunk; ++k)
+                  if (c0 + k < tan) row[k] *= sc[k];
+              }
+            } else {
+              double acc[kChunk];
+#pragma unroll
+              for (int k = 0; k < kChunk; ++k) acc[k] = 0.0;
+              for (int r = 0; r < w.kres; ++r) {
+                const double* row = v + static_cast<size_t>(r) * rs + c0;
+                const double wr = kOp == kOpLeft ? x[row0 + r] : 0.0;
+#pragma unroll
+                for (int k = 0; k < kChunk; ++k) {
+                  const double a = c0 + k < tan ? row[k] : 0.0;
+                  acc[k] = fma(a, kOp == kOpLeft ? wr : a, acc[k]);
+                }
+              }
 #pragma unroll
               for (int k = 0; k < kChunk; ++k)
-                if (c0 + k < tan) row[k] *= sc[k];
+                if (c0 + k < tan) RedAddF64(y + col + c0 + k, acc[k]);
             }
-          } else {
-            double acc[kChunk];
-#pragma unroll
-            for (int k = 0; k < kChunk; ++k) acc[k] = 0.0;
-            for (int r = 0; r < w.kres; ++r) {
-              const double* row = v + static_cast<size_t>(r) * rs + c0;
-              const double wr = kOp == kOpLeft ? x[row0 + r] : 0.0;
-#pragma unroll
-              for (int k = 0; k < kChunk; ++k) {
-                const double a = c0 + k < tan ? row[k] : 0.0;
-                acc[k] = fma(a, kOp == kOpLeft ? wr : a, acc[k]);
-              }
-            }
-#pragma unroll
-            for (int k = 0; k < kChunk; ++k)
-              if (c0 + k < tan) RedAddF64(y + col + c0 + k, acc[k]);
           }
         }
       }
@@ -742,6 +768,154 @@ __global__ void __launch_bounds__(256) CgModelKernel(int n, const double* __rest
   FinishScalars<2>(red, v, S, slot);
 }
 
+// ---- block-Jacobi preconditioner: one thread per active parameter block b (pb_table row b:
+// delta_offset, tangent t), whose t x t blocks are packed upper triangles at block_offset[col].
+// Sizes are runtime values and the blocks stay in global memory, so any tangent size works.
+
+// inverse = (matrix + diag(d2))^-1 per block: Cholesky M = U'U in place, U^-1 in place, then
+// U^-1 U^-T in place.  A block whose pivot is not positive, not finite or lost to cancellation
+// (a camera seen once has a rank-2 block; d2 may be NULL) gets the scalar preconditioner's
+// diagonal 1 / (colnorm + d2) (1 where that is not finite) and zero off the diagonal.
+__global__ void __launch_bounds__(256) BlockJacobiFactorKernel(
+    int num_blocks, const int32_t* __restrict__ pb_table, const int32_t* __restrict__ block_offset,
+    const double* __restrict__ matrix, const double* __restrict__ colnorm,
+    const double* __restrict__ d2, double* __restrict__ inverse) {
+  constexpr double kPivotTolerance = 64 * 2.220446049250313e-16;
+  for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < num_blocks;
+       b += gridDim.x * blockDim.x) {
+    const int col = pb_table[8 * b + 1], t = pb_table[8 * b + 2];
+    if (col < 0 || t <= 0) continue;
+    const int off = block_offset[col];
+    const double* __restrict__ B = matrix + off;
+    double* __restrict__ M = inverse + off;
+    const int count = t * (t + 1) / 2;
+    for (int k = 0; k < count; ++k) M[k] = B[k];
+    for (int a = 0; a < t; ++a) M[PackedUpper(a, a, t)] += d2 ? d2[col + a] : 0.0;
+    bool ok = true;
+    for (int k = 0; k < t && ok; ++k) {
+      const double mkk = M[PackedUpper(k, k, t)];
+      double d = mkk;
+      for (int i = 0; i < k; ++i) d -= M[PackedUpper(i, k, t)] * M[PackedUpper(i, k, t)];
+      if (!(d > kPivotTolerance * mkk) || !isfinite(d)) {
+        ok = false;
+        break;
+      }
+      const double ukk = sqrt(d);
+      M[PackedUpper(k, k, t)] = ukk;
+      for (int j = k + 1; j < t; ++j) {
+        double s = M[PackedUpper(k, j, t)];
+        for (int i = 0; i < k; ++i) s -= M[PackedUpper(i, k, t)] * M[PackedUpper(i, j, t)];
+        M[PackedUpper(k, j, t)] = s / ukk;
+      }
+    }
+    if (!ok) {
+      for (int a = 0; a < t; ++a) {
+        const double m = 1.0 / (colnorm[col + a] + (d2 ? d2[col + a] : 0.0));
+        for (int c = a; c < t; ++c) M[PackedUpper(a, c, t)] = c == a ? (isfinite(m) ? m : 1.0) : 0.0;
+      }
+      continue;
+    }
+    // U^-1 column by column: entry (i, j) reads row i of U^-1 left of j and rows >= i of U's
+    // column j, so rows are overwritten in ascending order and the diagonal last
+    for (int j = 0; j < t; ++j) {
+      const double ujj = M[PackedUpper(j, j, t)];
+      for (int i = 0; i < j; ++i) {
+        double s = 0.0;
+        for (int k = i; k < j; ++k) s += M[PackedUpper(i, k, t)] * M[PackedUpper(k, j, t)];
+        M[PackedUpper(i, j, t)] = -s / ujj;
+      }
+      M[PackedUpper(j, j, t)] = 1.0 / ujj;
+    }
+    // (U^-1 U^-T)(a, c) = sum_{k >= c} U^-1(a, k) U^-1(c, k), a <= c: in row-major order an
+    // entry is written after every read of it
+    for (int a = 0; a < t; ++a) {
+      for (int c = a; c < t; ++c) {
+        double s = 0.0;
+        for (int k = c; k < t; ++k) s += M[PackedUpper(a, k, t)] * M[PackedUpper(c, k, t)];
+        M[PackedUpper(a, c, t)] = s;
+      }
+    }
+  }
+}
+
+// r = b;  x = 0;  rnorm2 = r.r  (z, rho and p follow from CgBlockApplyKernel)
+__global__ void __launch_bounds__(256) CgBlockInitKernel(int n, const double* __restrict__ b,
+                                                         double* r, double* x, double* S,
+                                                         const ScalarReduce red) {
+  double rr = 0.0;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const double ri = b[i];
+    r[i] = ri;
+    x[i] = 0.0;
+    rr += ri * ri;
+  }
+  const double v[1] = {BlockSum(rr)};
+  const int slot[1] = {kSRnorm2};
+  FinishScalars<1>(red, v, S, slot);
+}
+
+// alpha = rho / pq;  x += alpha p;  r -= alpha (q + d2 p);  |r|^2 and x.(b + r) into Snext
+__global__ void __launch_bounds__(256) CgBlockUpdateKernel(int n, const double* __restrict__ p,
+                                                           const double* __restrict__ q,
+                                                           const double* __restrict__ d2,
+                                                           const double* __restrict__ b, double* x,
+                                                           double* r, const double* S,
+                                                           double* Snext, const ScalarReduce red) {
+  const double alpha = S[kSRho] / S[kSPq];
+  double rr = 0.0, xbr = 0.0;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const double pi = p[i];
+    const double xi = x[i] + alpha * pi;
+    const double ri = r[i] - alpha * (q[i] + (d2 ? d2[i] : 0.0) * pi);
+    x[i] = xi;
+    r[i] = ri;
+    rr += ri * ri;
+    xbr += xi * (b[i] + ri);
+  }
+  const double v[2] = {BlockSum(rr), BlockSum(xbr)};
+  const int slot[2] = {kSRnorm2, kSXbr};
+  FinishScalars<2>(red, v, Snext, slot);
+}
+
+// z_b = inverse_b r_b per parameter block;  rho = r.z into S
+__global__ void __launch_bounds__(256) CgBlockApplyKernel(
+    int num_blocks, const int32_t* __restrict__ pb_table, const int32_t* __restrict__ block_offset,
+    const double* __restrict__ inverse, const double* __restrict__ r, double* __restrict__ z,
+    double* S, const ScalarReduce red) {
+  double rho = 0.0;
+  for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < num_blocks;
+       b += gridDim.x * blockDim.x) {
+    const int col = pb_table[8 * b + 1], t = pb_table[8 * b + 2];
+    if (col < 0 || t <= 0) continue;
+    const double* __restrict__ M = inverse + block_offset[col];
+    const double* __restrict__ rb = r + col;
+    for (int a = 0; a < t; ++a) {
+      double acc = 0.0;
+      for (int c = 0; c < t; ++c)
+        acc = fma(M[a <= c ? PackedUpper(a, c, t) : PackedUpper(c, a, t)], rb[c], acc);
+      z[col + a] = acc;
+      rho = fma(rb[a], acc, rho);
+    }
+  }
+  const double v[1] = {BlockSum(rho)};
+  const int slot[1] = {kSRho};
+  FinishScalars<1>(red, v, S, slot);
+}
+
+// p = z + (rho_next / rho) p
+__global__ void __launch_bounds__(256) CgBlockDirectionKernel(int n, const double* __restrict__ z,
+                                                              double* p, const double* S,
+                                                              const double* Snext) {
+  const double beta = Snext[kSRho] / S[kSRho];
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    p[i] = z[i] + beta * p[i];
+}
+
+__global__ void __launch_bounds__(256) FillKernel(int n, double value, double* __restrict__ out) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    out[i] = value;
+}
+
 // ---- trust-region vector kernels (state, step and diagonals resident in HBM)
 __global__ void __launch_bounds__(256) JacobiScaleKernel(int n, const double* __restrict__ colnorm,
                                                          double* __restrict__ scale) {
@@ -914,6 +1088,15 @@ struct cb200_engine {
   // scaling): computed once per evaluation - by the scaling pass itself where the per-type
   // kernel runs - and shared by the LM diagonal and the conjugate-gradient preconditioner.
   bool colnorm_valid = false;
+  // Block-Jacobi preconditioner (allocated on first use): bj_offset[c] is where the packed
+  // upper triangle of the parameter block whose first column is c starts (blocks in column
+  // order; -1 for other columns).  bj_matrix = blockdiag(J'J) of the values as they stand,
+  // valid together with colnorm_valid's values; bj_inverse = (blockdiag(J'J) + D^2)^-1 of the
+  // last solve.
+  DeviceBuffer<int32_t> bj_offset;
+  DeviceBuffer<double> bj_matrix, bj_inverse;
+  int64_t bj_size = -1;             // doubles of bj_matrix; -1: table not built yet
+  bool bj_valid = false;
   bool plus_on_device = true;       // every manifold of the program is one PlusKernel knows
 
   void* comm = nullptr;
@@ -996,6 +1179,7 @@ void cb200_engine_destroy(cb200_engine* e) {
     delete t;
   }
   for (auto& b : e->la_col) b.Free();
+  e->bj_offset.Free(); e->bj_matrix.Free(); e->bj_inverse.Free();
   e->la_row.Free(); e->la_scalars.Free(); e->la_partials.Free(); e->la_arrivals.Free();
   for (auto& b : e->tr_state) b.Free();
   e->tr_scale.Free(); e->tr_diagonal.Free(); e->tr_delta.Free();
@@ -1573,7 +1757,7 @@ static int EvaluateOnDevice(cb200_engine* e, uint32_t flags, bool want_r, bool w
                             bool want_j) {
   cudaStream_t s = e->stream;
   if (want_j) e->jacobian_resident = true;   // values of an older evaluation are overwritten
-  if (want_j) e->colnorm_valid = false;
+  if (want_j) e->colnorm_valid = e->bj_valid = false;
   if (want_r) e->residuals_resident = true;
   CB200_CUDA(e, cudaMemsetAsync(e->d_status.ptr, 0, 2 * sizeof(int32_t), s));
   const size_t ne = static_cast<size_t>(e->num_effective);
@@ -1859,6 +2043,7 @@ static int RunJacobianWalk(cb200_engine* e, int op, const double* x, double* y) 
     w.jstride = t->d_jstride.ptr;
     w.respos = t->d_respos.ptr;
     w.pb_table = e->d_pb_table.ptr;
+    w.block_offset = e->bj_offset.ptr;
     w.values = e->d_jacobian.ptr;
     const int grid = std::min((t->n_local + 255) / 256, 148 * 16);
     // The per-type kernel (compile-time sizes, coalesced cell runs: ceres/internal/
@@ -1911,6 +2096,9 @@ static int RunJacobianWalk(cb200_engine* e, int op, const double* x, double* y) 
       case kOpRight: JacobianWalkKernel<kOpRight><<<grid, 256, 0, s>>>(w, x, y); break;
       case kOpLeft: JacobianWalkKernel<kOpLeft><<<grid, 256, 0, s>>>(w, x, y); break;
       case kOpColumnNorm: JacobianWalkKernel<kOpColumnNorm><<<grid, 256, 0, s>>>(w, x, y); break;
+      case kOpBlockDiagonal:
+        JacobianWalkKernel<kOpBlockDiagonal><<<grid, 256, 0, s>>>(w, x, y);
+        break;
       case kOpScaleNorm:
         JacobianWalkKernel<kOpScale><<<grid, 256, 0, s>>>(w, x, nullptr);
         JacobianWalkKernel<kOpColumnNorm><<<grid, 256, 0, s>>>(w, nullptr, y);
@@ -2017,7 +2205,7 @@ int cb200_engine_jacobian_squared_column_norm(cb200_engine* e, double* out) {
 }
 
 int cb200_engine_jacobian_scale_columns(cb200_engine* e, const double* scale) {
-  if (e) e->colnorm_valid = false;
+  if (e) e->colnorm_valid = e->bj_valid = false;
   NvtxRange nvtx_range("cb200_engine_jacobian_scale_columns");
   int rc = PrepareLinearAlgebra(e, false);
   if (rc != CB200_OK) return rc;
@@ -2031,6 +2219,35 @@ int cb200_engine_jacobian_scale_columns(cb200_engine* e, const double* scale) {
   return CB200_OK;
 }
 
+// Block-Jacobi storage on first use: the active parameter blocks in column order, each a packed
+// upper triangle, found through bj_offset by its first column.
+static int PrepareBlockJacobi(cb200_engine* e) {
+  if (e->bj_size >= 0) return CB200_OK;
+  std::vector<std::pair<int32_t, int32_t>> blocks;  // (first column, tangent size)
+  for (int32_t b = 0; b < e->num_active; ++b)
+    if (e->blocks[b].delta_offset >= 0 && e->blocks[b].tangent_size > 0)
+      blocks.emplace_back(e->blocks[b].delta_offset, e->blocks[b].tangent_size);
+  // program order is usually column order already; sorting 4.5 M blocks costs ~0.2 s
+  if (!std::is_sorted(blocks.begin(), blocks.end())) std::sort(blocks.begin(), blocks.end());
+  std::vector<int32_t> table(static_cast<size_t>(e->num_effective) + 1, -1);
+  int64_t total = 0;
+  for (const auto& b : blocks) {
+    if (total > INT32_MAX)
+      return e->Fail(CB200_ERROR_INVALID_ARGUMENT,
+                     "block-Jacobi preconditioner: %lld packed entries exceed the 32-bit offsets",
+                     static_cast<long long>(total));
+    table[b.first] = static_cast<int32_t>(total);
+    total += static_cast<int64_t>(b.second) * (b.second + 1) / 2;
+  }
+  CB200_CUDA(e, e->bj_offset.Upload(table, e->stream));
+  CB200_CUDA(e, e->bj_matrix.Resize(static_cast<size_t>(total) + 1));
+  CB200_CUDA(e, e->bj_inverse.Resize(static_cast<size_t>(total) + 1));
+  CB200_CUDA(e, cudaStreamSynchronize(e->stream));  // `table` dies at scope end
+  e->bj_size = total;
+  e->bj_valid = false;
+  return CB200_OK;
+}
+
 // The solve itself.  d_squared: host pointer (copied in), or with d_squared_on_device the
 // LM diagonal already in la_col[6]; the solution stays in la_col[0] and is copied to
 // `solution` when that is not NULL.
@@ -2041,6 +2258,13 @@ static int CgnrSolve(cb200_engine* e, const double* d_squared, bool d_squared_on
   if (rc != CB200_OK) return rc;
   if (!options || !summary)
     return e->Fail(CB200_ERROR_INVALID_ARGUMENT, "options and summary are required");
+  const int preconditioner = options->preconditioner;
+  if (preconditioner != CB200_PRECONDITIONER_SCALAR_JACOBI &&
+      preconditioner != CB200_PRECONDITIONER_BLOCK_JACOBI &&
+      preconditioner != CB200_PRECONDITIONER_IDENTITY)
+    return e->Fail(CB200_ERROR_INVALID_ARGUMENT, "unknown preconditioner %d", preconditioner);
+  const bool block = preconditioner == CB200_PRECONDITIONER_BLOCK_JACOBI;
+  if (block && (rc = PrepareBlockJacobi(e)) != CB200_OK) return rc;
   cudaStream_t s = e->stream;
   const int ne = e->num_effective, m = e->res_end - e->res_begin;
   const size_t col_bytes = static_cast<size_t>(ne) * sizeof(double);
@@ -2053,6 +2277,7 @@ static int CgnrSolve(cb200_engine* e, const double* d_squared, bool d_squared_on
   double* S = e->la_scalars.ptr;  // three rotating sets of scalars
   const int vgrid = std::max(1, std::min((ne + 255) / 256, kMaxVectorGrid));
   const int rgrid = std::max(1, std::min((m + 255) / 256, kMaxVectorGrid));
+  const int bgrid = std::max(1, std::min((e->num_active + 255) / 256, kMaxVectorGrid));
   const ScalarReduce red{e->la_partials.ptr, e->la_arrivals.ptr};
   std::memset(summary, 0, sizeof(*summary));
   bool one_pass = true;
@@ -2073,7 +2298,31 @@ static int CgnrSolve(cb200_engine* e, const double* d_squared, bool d_squared_on
     e->colnorm_valid = true;
   }
   CB200_CUDA(e, cudaMemsetAsync(S, 0, 3 * kSCount * sizeof(double), s));
-  CgInitKernel<<<vgrid, 256, 0, s>>>(ne, colnorm, d2, b, minv, r, p, x, S, red);
+  if (block) {
+    // blockdiag(J'J) once per Jacobian (a rejected step reuses it), its damped inverse per
+    // solve; minv holds z = M^-1 r
+    if (!e->bj_valid) {
+      const size_t bytes = static_cast<size_t>(e->bj_size) * sizeof(double);
+      CB200_CUDA(e, cudaMemsetAsync(e->bj_matrix.ptr, 0, bytes, s));
+      if ((rc = RunJacobianWalk(e, kOpBlockDiagonal, nullptr, e->bj_matrix.ptr)) != CB200_OK)
+        return rc;
+      if ((rc = SumOverRanks(e, e->bj_matrix.ptr, e->bj_size)) != CB200_OK) return rc;
+      e->bj_valid = true;
+    }
+    BlockJacobiFactorKernel<<<bgrid, 256, 0, s>>>(e->num_active, e->d_pb_table.ptr,
+                                                   e->bj_offset.ptr, e->bj_matrix.ptr, colnorm,
+                                                   d2, e->bj_inverse.ptr);
+    CgBlockInitKernel<<<vgrid, 256, 0, s>>>(ne, b, r, x, S, red);
+    CgBlockApplyKernel<<<bgrid, 256, 0, s>>>(e->num_active, e->d_pb_table.ptr, e->bj_offset.ptr,
+                                              e->bj_inverse.ptr, r, minv, S, red);
+    CB200_CUDA(e, cudaMemcpyAsync(p, minv, col_bytes, cudaMemcpyDeviceToDevice, s));
+  } else if (preconditioner == CB200_PRECONDITIONER_IDENTITY) {
+    // the scalar kernels with minv = 1 / (1 + 0); q is rewritten before its first use
+    FillKernel<<<vgrid, 256, 0, s>>>(ne, 1.0, q);
+    CgInitKernel<<<vgrid, 256, 0, s>>>(ne, q, nullptr, b, minv, r, p, x, S, red);
+  } else {
+    CgInitKernel<<<vgrid, 256, 0, s>>>(ne, colnorm, d2, b, minv, r, p, x, S, red);
+  }
   CB200_CUDA(e, cudaMemcpyAsync(e->h_la_scalars, S, kSCount * sizeof(double),
                                 cudaMemcpyDeviceToHost, s));
   CB200_CUDA(e, cudaStreamSynchronize(s));
@@ -2101,8 +2350,16 @@ static int CgnrSolve(cb200_engine* e, const double* d_squared, bool d_squared_on
       if ((rc = SumOverRanks(e, q, ne)) != CB200_OK) return rc;
       CgDotKernel<<<vgrid, 256, 0, s>>>(ne, p, q, d2, Sc, red);
       CB200_CUDA(e, cudaMemsetAsync(Sn, 0, kSCount * sizeof(double), s));
-      CgUpdateKernel<<<vgrid, 256, 0, s>>>(ne, p, q, d2, minv, b, x, r, Sc, Sn, red);
-      CgDirectionKernel<<<vgrid, 256, 0, s>>>(ne, r, minv, p, Sc, Sn);
+      if (block) {
+        CgBlockUpdateKernel<<<vgrid, 256, 0, s>>>(ne, p, q, d2, b, x, r, Sc, Sn, red);
+        CgBlockApplyKernel<<<bgrid, 256, 0, s>>>(e->num_active, e->d_pb_table.ptr,
+                                                  e->bj_offset.ptr, e->bj_inverse.ptr, r, minv,
+                                                  Sn, red);
+        CgBlockDirectionKernel<<<vgrid, 256, 0, s>>>(ne, minv, p, Sc, Sn);
+      } else {
+        CgUpdateKernel<<<vgrid, 256, 0, s>>>(ne, p, q, d2, minv, b, x, r, Sc, Sn, red);
+        CgDirectionKernel<<<vgrid, 256, 0, s>>>(ne, r, minv, p, Sc, Sn);
+      }
       CB200_CUDA(e, cudaMemcpyAsync(e->h_la_scalars, S, 3 * kSCount * sizeof(double),
                                     cudaMemcpyDeviceToHost, s));
       CB200_CUDA(e, cudaStreamSynchronize(s));
@@ -2224,6 +2481,7 @@ int cb200_engine_jacobi_scale(cb200_engine* e, int compute) {
   cudaStream_t s = e->stream;
   const int ne = e->num_effective;
   const int grid = std::max(1, std::min((ne + 255) / 256, kMaxVectorGrid));
+  e->bj_valid = false;  // the values are scaled below
   if (compute) {
     double* col = e->la_col[7].ptr;
     CB200_CUDA(e, cudaMemsetAsync(col, 0, static_cast<size_t>(ne) * sizeof(double), s));

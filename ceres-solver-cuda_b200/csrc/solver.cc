@@ -140,6 +140,13 @@ bool Solver::Options::IsValid(std::string* error) const {
     return false;
   }
   if (max_num_iterations < 0) { *error = "max_num_iterations < 0"; return false; }
+  // only the conjugate gradients on the device-resident Jacobian read the preconditioner
+  if (preconditioner_type != SCALAR_JACOBI &&
+      (linear_solver_type != CGNR || sparse_linear_algebra_library_type != CUDA_SPARSE)) {
+    *error = "preconditioner_type IDENTITY and JACOBI require linear_solver_type = CGNR and "
+             "sparse_linear_algebra_library_type = CUDA_SPARSE.";
+    return false;
+  }
   return true;
 }
 
@@ -200,8 +207,13 @@ enum Result { kDone, kRejected, kError };
 // levenberg_marquardt_strategy.cc:97-118: inexact step, stopped by the relative decrease of
 // the quadratic model (eta) and not by the residual (r_tolerance = -1)
 cb200_cgnr_options ConjugateGradientOptions(const Solver::Options& options) {
+  const int32_t preconditioner = options.preconditioner_type == JACOBI
+                                     ? CB200_PRECONDITIONER_BLOCK_JACOBI
+                                 : options.preconditioner_type == IDENTITY
+                                     ? CB200_PRECONDITIONER_IDENTITY
+                                     : CB200_PRECONDITIONER_SCALAR_JACOBI;
   return {options.min_linear_solver_iterations, options.max_linear_solver_iterations, -1.0,
-          options.eta};
+          options.eta, preconditioner};
 }
 
 class TrustRegionState {

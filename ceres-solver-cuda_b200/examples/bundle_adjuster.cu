@@ -5,6 +5,7 @@
 //
 //   bundle_adjuster --input=problem.txt [--robustify] [--num_iterations=20]
 //                   [--linear_solver=iterative_schur|cgnr|cgnr_cuda] [--constant_first_camera]
+//                   [--preconditioner=identity|jacobi|scalar_jacobi]   (cgnr_cuda only)
 //   bundle_adjuster --synthetic=16,2000,8000 ...
 //   bundle_adjuster --input=problem.txt --check_input     (parse only, no GPU needed)
 //
@@ -94,7 +95,8 @@ int main(int argc, char** argv) {
     bal.Synthesize(nc, np, nobs, 1);
   } else {
     std::fprintf(stderr, "usage: %s --input=<bal file> | --synthetic=nc,np,nobs [--robustify] "
-                 "[--num_iterations=N] [--linear_solver=iterative_schur|cgnr|cgnr_cuda] [--bulk]\n", argv[0]);
+                 "[--num_iterations=N] [--linear_solver=iterative_schur|cgnr|cgnr_cuda] [--bulk] "
+                 "[--preconditioner=identity|jacobi|scalar_jacobi]\n", argv[0]);
     return 1;
   }
   if (Flag(argc, argv, "--check_input")) {
@@ -163,6 +165,18 @@ int main(int argc, char** argv) {
     // the Jacobian never leaves the device: evaluation and conjugate gradients both run there
     options.linear_solver_type = ceres::CGNR;
     options.sparse_linear_algebra_library_type = ceres::CUDA_SPARSE;
+  }
+  if (const char* pc = Flag(argc, argv, "--preconditioner")) {
+    if (!std::strcmp(pc, "identity")) {
+      options.preconditioner_type = ceres::IDENTITY;
+    } else if (!std::strcmp(pc, "jacobi")) {
+      options.preconditioner_type = ceres::JACOBI;
+    } else if (!std::strcmp(pc, "scalar_jacobi")) {
+      options.preconditioner_type = ceres::SCALAR_JACOBI;
+    } else {
+      std::fprintf(stderr, "unknown --preconditioner=%s\n", pc);
+      return 1;
+    }
   }
   // The points come before the cameras.
   auto* ordering = new ceres::ParameterBlockOrdering;

@@ -87,6 +87,10 @@ class Solver {
     double parameter_tolerance = 1e-8;
     LinearSolverType linear_solver_type = SPARSE_NORMAL_CHOLESKY;
     SparseLinearAlgebraLibraryType sparse_linear_algebra_library_type = NO_SPARSE;
+    // IDENTITY and JACOBI need CGNR with CUDA_SPARSE.  The default is SCALAR_JACOBI rather
+    // than Ceres' JACOBI so that existing callers keep the steps they had before this option
+    // existed.
+    PreconditionerType preconditioner_type = SCALAR_JACOBI;
     std::shared_ptr<ParameterBlockOrdering> linear_solver_ordering;
     int min_linear_solver_iterations = 0;
     int max_linear_solver_iterations = 500;

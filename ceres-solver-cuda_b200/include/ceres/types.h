@@ -28,6 +28,15 @@ enum SparseLinearAlgebraLibraryType {
   NO_SPARSE
 };
 
+// Preconditioner of the iterative linear solvers; this library reads it for CGNR with
+// CUDA_SPARSE (the conjugate gradients on the device-resident Jacobian).
+//   IDENTITY       no preconditioning.
+//   JACOBI         the block diagonal of J'J + D'D, one dense block per parameter block,
+//                  inverted (Ceres' CGNR JACOBI).
+//   SCALAR_JACOBI  extension of this library, not a Ceres name: the scalar diagonal
+//                  diag(J'J + D'D)^-1.
+enum PreconditionerType { IDENTITY, JACOBI, SCALAR_JACOBI };
+
 enum MinimizerType { LINE_SEARCH, TRUST_REGION };
 
 constexpr int DYNAMIC = -1;

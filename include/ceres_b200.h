@@ -326,11 +326,20 @@ int cb200_engine_jacobian_squared_column_norm(cb200_engine* engine, double* out)
 /* J <- J diag(scale) */
 int cb200_engine_jacobian_scale_columns(cb200_engine* engine, const double* scale);
 
+/* Preconditioner M of the conjugate gradients, for A = J'J + diag(d_squared).  Zero is the
+ * scalar diagonal, so zero-initialised options keep it. */
+#define CB200_PRECONDITIONER_SCALAR_JACOBI 0 /* diag(A)^-1 (1 where a diagonal entry is not positive) */
+#define CB200_PRECONDITIONER_BLOCK_JACOBI 1  /* blockdiag(A)^-1: one dense tangent x tangent block per
+                                                parameter block (Ceres' CGNR JACOBI); a block whose
+                                                Cholesky factorisation breaks down uses the scalar rule */
+#define CB200_PRECONDITIONER_IDENTITY 2      /* none */
+
 typedef struct cb200_cgnr_options {
   int32_t min_num_iterations;
   int32_t max_num_iterations;
   double r_tolerance; /* stop when |residual| <= r_tolerance * |J'b|  (conjugate_gradients_solver.h) */
   double q_tolerance; /* stop when the relative decrease of the quadratic model falls below this */
+  int32_t preconditioner; /* CB200_PRECONDITIONER_* */
 } cb200_cgnr_options;
 
 typedef struct cb200_cgnr_summary {
@@ -345,8 +354,12 @@ typedef struct cb200_cgnr_summary {
 
 /* Solves (J'J + diag(d_squared)) y = J'b by preconditioned conjugate gradients on the
  * normal equations without forming them, b = the residuals of the last evaluation (on the
- * device) and J its Jacobian (CB200_KEEP_*_ON_DEVICE), preconditioner
- * diag(J'J + d_squared)^-1.  d_squared may be NULL (zero).  solution: num_effective doubles. */
+ * device) and J its Jacobian (CB200_KEEP_*_ON_DEVICE), preconditioner options->preconditioner.
+ * The block-Jacobi preconditioner keeps blockdiag(J'J) (packed upper triangles, in column order)
+ * and its inverse in HBM, about 2 x 8 x sum(tangent * (tangent + 1) / 2) bytes; blockdiag(J'J) is
+ * computed once per Jacobian and reused until an evaluation, a column scaling or
+ * cb200_engine_jacobi_scale changes the values.  d_squared may be NULL (zero).  solution:
+ * num_effective doubles. */
 int cb200_engine_cgnr_solve(cb200_engine* engine, const double* d_squared,
                             const cb200_cgnr_options* options, double* solution,
                             cb200_cgnr_summary* summary);

@@ -54,6 +54,12 @@ for fmt, kw in ((0, {}), (1, {"subset_manifold": True})):
     print(f"rank {rank}/{world} fmt {fmt}: device linear algebra {e_la:.1e}, 30 CG iterations {e_cg:.1e} "
           f"({s1['ms'] / 30:.3f} ms/iteration sharded, {s0['ms'] / 30:.3f} unsharded) "
           f"{'OK' if e_la <= 1e-11 and e_cg <= 1e-8 else 'MISMATCH'}", flush=True)
+    # blockdiag(J'J) is summed over the ranks as well
+    y0, s0 = full.cgnr_solve(d2, max_iterations=30, r_tolerance=-1, q_tolerance=-1, preconditioner="jacobi")
+    y1, s1 = sh.cgnr_solve(d2, max_iterations=30, r_tolerance=-1, q_tolerance=-1, preconditioner="jacobi")
+    e_bj = max(rel(y1, y0), abs(s1["jy_dot_b"] - s0["jy_dot_b"]) / abs(s0["jy_dot_b"]))
+    print(f"rank {rank}/{world} fmt {fmt}: 30 block-Jacobi CG iterations {e_bj:.1e} "
+          f"{'OK' if e_bj <= 1e-8 else 'MISMATCH'}", flush=True)
     t = sh.timing()
     mode = {0: "single", 1: "nccl all-reduce", 2: "peer exchange"}[sh.exchange_mode()]
     # the other output combinations take the unfused path (PushExclusiveKernel)
