@@ -13,7 +13,8 @@ CXXFLAGS := -O2 -std=c++17 -fPIC -Wall -Wno-unknown-pragmas $(INC) -I/usr/local/
 LIB := $(PKG)/lib/libceres_b200.so
 DRV := tests/driver/libceres_b200_driver.so
 HDRS := $(wildcard include/*.h $(PKG)/include/ceres/*.h $(PKG)/include/ceres/internal/*.h $(PKG)/include/ceres/internal/*.cuh)
-DRV_SRCS := driver_api driver_bal driver_bal2 driver_pose driver_pose3d driver_tests driver_preconditioner
+DRV_SRCS := driver_api driver_bal driver_bal2 driver_pose driver_pose3d driver_tests driver_preconditioner \
+            driver_losses driver_losses2
 DRV_OBJS := $(patsubst %,build/driver/%.o,$(DRV_SRCS))
 
 EXAMPLE := build/examples/bundle_adjuster
@@ -36,7 +37,7 @@ $(LIB): build/engine.o build/host.o build/solver.o
 	@mkdir -p $(PKG)/lib
 	$(NVCC) $(ARCH) -shared -o $@ $^ -lcudart -ldl
 
-build/driver/%.o: tests/driver/%.cu tests/driver/driver.h tests/driver/test_functors.h $(HDRS) $(wildcard $(PKG)/examples/*.h)
+build/driver/%.o: tests/driver/%.cu $(wildcard tests/driver/*.h) $(HDRS) $(wildcard $(PKG)/examples/*.h)
 	@mkdir -p build/driver
 	$(NVCC) $(NVFLAGS) -I$(PKG)/examples -Itests/driver -Xptxas -v -c $< -o $@ 2> $@.ptxas.log || (cat $@.ptxas.log; false)
 

@@ -10,6 +10,8 @@ import subprocess
 
 import numpy as np
 
+from . import problems as P
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB_PATH = os.path.join(ROOT, "ceres-solver-cuda_b200", "lib", "libceres_b200.so")
 DRIVER_PATH = os.path.join(ROOT, "tests", "driver", "libceres_b200_driver.so")
@@ -133,8 +135,40 @@ def driver():
         L.drv_options_is_valid_for.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                                C.c_char_p, C.c_int]
         L.drv_argument_slot_ordering.argtypes = [C.c_void_p, C.c_void_p]
+        L.drv_loss_evaluate.argtypes = [C.c_int, C.c_double, C.c_double, C.c_double, C.c_void_p]
+        L.drv_add_residual_blocks.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 6 + \
+            [C.c_int, C.c_int, C.c_void_p, C.c_void_p]
+        L.drv_composed_loss_evaluate.argtypes = [C.c_int, C.c_double, C.c_double, C.c_double,
+                                                 C.c_void_p]
         _DRV = L
     return _DRV
+
+
+def _create(spec, bulk):
+    """drv_create for a ProblemSpec.  Specs with the loss kinds of driver_losses.h
+    (problems.LOSS_SOFT_L1 and up) get their parameter blocks from drv_create and their residual
+    blocks from drv_add_residual_blocks; the problem is the same one either way."""
+    L = driver()
+    if not (spec.rb_loss_kind >= P.LOSS_SOFT_L1).any():
+        return L.drv_create(
+            spec.num_pb, _p(spec.pb_size), _p(spec.pb_values), _p(spec.pb_constant),
+            _p(spec.pb_manifold_kind), _p(spec.pb_manifold_param), spec.num_rb,
+            _p(spec.rb_type), _p(spec.rb_pb), _p(spec.rb_loss_kind), _p(spec.rb_loss_a),
+            _p(spec.rb_loss_b), _p(spec.fdata), int(bulk))
+    h = L.drv_create(
+        spec.num_pb, _p(spec.pb_size), _p(spec.pb_values), _p(spec.pb_constant),
+        _p(spec.pb_manifold_kind), _p(spec.pb_manifold_param), 0, None, None, None, None, None,
+        None, int(bulk))
+    num_types = max(P.COST_TYPES) + 1
+    blocks = np.zeros(num_types, dtype=np.int32)
+    flen = np.zeros(num_types, dtype=np.int32)
+    for t, (_, sizes, n) in P.COST_TYPES.items():
+        blocks[t], flen[t] = len(sizes), n
+    L.drv_add_residual_blocks(
+        h, spec.num_rb, _p(spec.rb_type), _p(spec.rb_pb), _p(spec.rb_loss_kind),
+        _p(spec.rb_loss_a), _p(spec.rb_loss_b), _p(spec.fdata), int(bulk) & 1, num_types,
+        _p(blocks), _p(flen))
+    return h
 
 
 def nccl_unique_id() -> bytes:
@@ -178,11 +212,7 @@ def solve(spec, linear_solver_type=ITERATIVE_SCHUR, max_num_iterations=20, order
     and the solution in the specification's parameter-block order.  preconditioner: a key of
     PRECONDITIONERS (Solver::Options::preconditioner_type)."""
     L = driver()
-    h = L.drv_create(
-        spec.num_pb, _p(spec.pb_size), _p(spec.pb_values), _p(spec.pb_constant),
-        _p(spec.pb_manifold_kind), _p(spec.pb_manifold_param), spec.num_rb,
-        _p(spec.rb_type), _p(spec.rb_pb), _p(spec.rb_loss_kind), _p(spec.rb_loss_a),
-        _p(spec.rb_loss_b), _p(spec.fdata), int(bulk))
+    h = _create(spec, int(bulk))
     err = L.drv_error(h)
     if err:
         raise RuntimeError(err.decode())
@@ -207,11 +237,7 @@ def argument_slot_ordering(spec):
     """internal::ArgumentSlotOrdering on the ProblemSpec (host code, no GPU): (found, group per
     parameter block)."""
     L = driver()
-    h = L.drv_create(
-        spec.num_pb, _p(spec.pb_size), _p(spec.pb_values), _p(spec.pb_constant),
-        _p(spec.pb_manifold_kind), _p(spec.pb_manifold_param), spec.num_rb,
-        _p(spec.rb_type), _p(spec.rb_pb), _p(spec.rb_loss_kind), _p(spec.rb_loss_a),
-        _p(spec.rb_loss_b), _p(spec.fdata), 0)
+    h = _create(spec, 0)
     err = L.drv_error(h)
     if err:
         raise RuntimeError(err.decode())
@@ -221,16 +247,31 @@ def argument_slot_ordering(spec):
     return bool(found), groups
 
 
+def loss_evaluate(kind, a, b, s):
+    """[rho(s), rho'(s), rho''(s)] of the product's loss class for a loss kind (problems.LOSS_*)
+    with parameters a, b, evaluated on the host as Problem::EvaluateResidualBlock does."""
+    rho = np.zeros(3)
+    if not driver().drv_loss_evaluate(int(kind), float(a), float(b), float(s), _p(rho)):
+        raise ValueError(f"loss kind {kind} has no loss object")
+    return rho
+
+
+def composed_loss_evaluate(which, a, b, s):
+    """Host evaluation of ComposedLossCUDA<HuberLossCUDA, CauchyLossCUDA>(Huber(a), Cauchy(b))
+    (which = 0) or ComposedLossCUDA<TolerantLossCUDA, TukeyLossCUDA>(Tolerant(a, b), Tukey(a))
+    (which = 1)."""
+    rho = np.zeros(3)
+    if not driver().drv_composed_loss_evaluate(int(which), float(a), float(b), float(s), _p(rho)):
+        raise ValueError(f"no composition {which}")
+    return rho
+
+
 def options_is_valid(spec, minimizer_type, linear_solver_type=None, cuda_sparse=False,
                      preconditioner=None):
     """Solver::Options::IsValid with use_cuda_for_evaluator (reference solver.cc:702-708);
     None keeps an option's default.  Returns (valid, message)."""
     L = driver()
-    h = L.drv_create(
-        spec.num_pb, _p(spec.pb_size), _p(spec.pb_values), _p(spec.pb_constant),
-        _p(spec.pb_manifold_kind), _p(spec.pb_manifold_param), spec.num_rb,
-        _p(spec.rb_type), _p(spec.rb_pb), _p(spec.rb_loss_kind), _p(spec.rb_loss_a),
-        _p(spec.rb_loss_b), _p(spec.fdata), 0)
+    h = _create(spec, 0)
     msg = C.create_string_buffer(512)
     ok = L.drv_options_is_valid_for(
         h, int(minimizer_type), -1 if linear_solver_type is None else int(linear_solver_type),
@@ -254,11 +295,7 @@ class CudaProblem:
         if bulk is None:
             bulk = spec.num_rb > 5000
         bulk = int(bool(bulk)) | (2 if evaluation_callback else 0)
-        self.h = L.drv_create(
-            spec.num_pb, _p(spec.pb_size), _p(spec.pb_values), _p(spec.pb_constant),
-            _p(spec.pb_manifold_kind), _p(spec.pb_manifold_param), spec.num_rb,
-            _p(spec.rb_type), _p(spec.rb_pb), _p(spec.rb_loss_kind), _p(spec.rb_loss_a),
-            _p(spec.rb_loss_b), _p(spec.fdata), int(bulk))
+        self.h = _create(spec, int(bulk))
         err = L.drv_error(self.h)
         if err:
             raise RuntimeError(err.decode())

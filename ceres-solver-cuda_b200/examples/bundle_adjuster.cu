@@ -1,9 +1,10 @@
 // Bundle adjustment with the CUDA evaluator, written against the same API as the
 // reference's examples/bundle_adjuster.cu.cc (BuildProblem :302-366, SetOrdering :225-268,
 // SolveProblem :368-392): one AddResidualBlock<SnavelyReprojectionError, 2, 9, 3> per
-// observation, HuberLossCUDA when --robustify, points eliminated before cameras.
+// observation, HuberLossCUDA(1) when --robustify, points eliminated before cameras.
 //
 //   bundle_adjuster --input=problem.txt [--robustify] [--num_iterations=20]
+//                   [--loss=huber|cauchy|soft_l1|arctan|tolerant|tukey]   (scale 1)
 //                   [--linear_solver=iterative_schur|cgnr|cgnr_cuda] [--constant_first_camera]
 //                   [--preconditioner=identity|jacobi|scalar_jacobi]   (cgnr_cuda only)
 //   bundle_adjuster --synthetic=16,2000,8000 ...
@@ -16,6 +17,7 @@
 #include <cstdlib>
 #include <algorithm>
 #include <cstring>
+#include <memory>
 #include <random>
 #include <string>
 #include <thread>
@@ -85,6 +87,71 @@ static const char* Flag(int argc, char** argv, const char* name) {
   return nullptr;
 }
 
+// One residual block per observation, each with a copy of *loss (null: no loss).  bulk: all
+// observations in one call sharing one loss object, no heap object per residual block (the
+// reference's per-block objects make its preprocessor take 47 s on the 29 M-block problem,
+// README.md:186).
+template <typename Loss>
+void AddObservations(ceres::ProblemCUDA* problem, BalProblem& bal, bool bulk, const Loss* loss) {
+  if (bulk) {
+    ceres::Problem::Options problem_options;
+    problem_options.loss_function_ownership = ceres::DO_NOT_TAKE_OWNERSHIP;
+    *problem = ceres::ProblemCUDA(problem_options);
+    static std::unique_ptr<Loss> shared_loss;
+    if (loss) shared_loss.reset(new Loss(*loss));
+    std::vector<ceres::examples::SnavelyReprojectionError> functors;
+    std::vector<double*> blocks;
+    functors.reserve(bal.num_observations);
+    blocks.reserve(2 * static_cast<size_t>(bal.num_observations));
+    for (int i = 0; i < bal.num_observations; ++i) {
+      functors.emplace_back(bal.observations[2 * i], bal.observations[2 * i + 1]);
+      blocks.push_back(&bal.cameras[9 * static_cast<size_t>(bal.camera_index[i])]);
+      blocks.push_back(&bal.points[3 * static_cast<size_t>(bal.point_index[i])]);
+    }
+    problem->AddResidualBlocks<ceres::examples::SnavelyReprojectionError, 2, 9, 3>(
+        bal.num_observations, functors.data(), shared_loss.get(), blocks.data());
+    return;
+  }
+  for (int i = 0; i < bal.num_observations; ++i) {
+    ceres::CostFunction* cost_function = ceres::examples::SnavelyReprojectionError::Create(
+        bal.observations[2 * i], bal.observations[2 * i + 1]);
+    double* camera = &bal.cameras[9 * static_cast<size_t>(bal.camera_index[i])];
+    double* point = &bal.points[3 * static_cast<size_t>(bal.point_index[i])];
+    problem->AddResidualBlock<ceres::examples::SnavelyReprojectionError, 2, 9, 3>(
+        cost_function, loss ? new Loss(*loss) : nullptr, camera, point);
+  }
+}
+
+// --loss=<name>: the loss of every residual block, all with scale 1 (Tolerant: a = b = 1).
+// Returns false for an unknown name.
+static bool AddObservations(ceres::ProblemCUDA* problem, BalProblem& bal, bool bulk,
+                            const char* loss) {
+  if (!loss) {
+    AddObservations(problem, bal, bulk, static_cast<const ceres::TrivialLossCUDA*>(nullptr));
+  } else if (!std::strcmp(loss, "huber")) {
+    const ceres::HuberLossCUDA l(1.0);
+    AddObservations(problem, bal, bulk, &l);
+  } else if (!std::strcmp(loss, "cauchy")) {
+    const ceres::CauchyLossCUDA l(1.0);
+    AddObservations(problem, bal, bulk, &l);
+  } else if (!std::strcmp(loss, "soft_l1")) {
+    const ceres::SoftLOneLossCUDA l(1.0);
+    AddObservations(problem, bal, bulk, &l);
+  } else if (!std::strcmp(loss, "arctan")) {
+    const ceres::ArctanLossCUDA l(1.0);
+    AddObservations(problem, bal, bulk, &l);
+  } else if (!std::strcmp(loss, "tolerant")) {
+    const ceres::TolerantLossCUDA l(1.0, 1.0);
+    AddObservations(problem, bal, bulk, &l);
+  } else if (!std::strcmp(loss, "tukey")) {
+    const ceres::TukeyLossCUDA l(1.0);
+    AddObservations(problem, bal, bulk, &l);
+  } else {
+    return false;
+  }
+  return true;
+}
+
 int main(int argc, char** argv) {
   BalProblem bal;
   if (const char* in = Flag(argc, argv, "--input")) {
@@ -95,6 +162,7 @@ int main(int argc, char** argv) {
     bal.Synthesize(nc, np, nobs, 1);
   } else {
     std::fprintf(stderr, "usage: %s --input=<bal file> | --synthetic=nc,np,nobs [--robustify] "
+                 "[--loss=huber|cauchy|soft_l1|arctan|tolerant|tukey] "
                  "[--num_iterations=N] [--linear_solver=iterative_schur|cgnr|cgnr_cuda] [--bulk] "
                  "[--preconditioner=identity|jacobi|scalar_jacobi]\n", argv[0]);
     return 1;
@@ -116,40 +184,13 @@ int main(int argc, char** argv) {
   const char* ls = Flag(argc, argv, "--linear_solver");
   const char* iters = Flag(argc, argv, "--num_iterations");
 
+  const char* loss = Flag(argc, argv, "--loss");
+  if (!loss && robustify) loss = "huber";
+
   ceres::ProblemCUDA problem;
-  static ceres::HuberLossCUDA shared_loss(1.0);
-  if (Flag(argc, argv, "--bulk")) {
-    // Beyond the reference: all observations in one call, no heap object per residual block
-    // (the reference's per-block objects make its preprocessor take 47 s on the 29 M-block
-    // problem, README.md:186).
-    ceres::Problem::Options problem_options;
-    problem_options.loss_function_ownership = ceres::DO_NOT_TAKE_OWNERSHIP;
-    problem = ceres::ProblemCUDA(problem_options);
-    std::vector<ceres::examples::SnavelyReprojectionError> functors;
-    std::vector<double*> blocks;
-    functors.reserve(bal.num_observations);
-    blocks.reserve(2 * static_cast<size_t>(bal.num_observations));
-    for (int i = 0; i < bal.num_observations; ++i) {
-      functors.emplace_back(bal.observations[2 * i], bal.observations[2 * i + 1]);
-      blocks.push_back(&bal.cameras[9 * static_cast<size_t>(bal.camera_index[i])]);
-      blocks.push_back(&bal.points[3 * static_cast<size_t>(bal.point_index[i])]);
-    }
-    if (robustify)
-      problem.AddResidualBlocks<ceres::examples::SnavelyReprojectionError, 2, 9, 3>(
-          bal.num_observations, functors.data(), &shared_loss, blocks.data());
-    else
-      problem.AddResidualBlocks<ceres::examples::SnavelyReprojectionError, 2, 9, 3>(
-          bal.num_observations, functors.data(), static_cast<ceres::TrivialLossCUDA*>(nullptr),
-          blocks.data());
-  } else
-  for (int i = 0; i < bal.num_observations; ++i) {
-    ceres::CostFunction* cost_function = ceres::examples::SnavelyReprojectionError::Create(
-        bal.observations[2 * i], bal.observations[2 * i + 1]);
-    ceres::HuberLossCUDA* loss_function = robustify ? new ceres::HuberLossCUDA(1.0) : nullptr;
-    double* camera = &bal.cameras[9 * static_cast<size_t>(bal.camera_index[i])];
-    double* point = &bal.points[3 * static_cast<size_t>(bal.point_index[i])];
-    problem.AddResidualBlock<ceres::examples::SnavelyReprojectionError, 2, 9, 3>(
-        cost_function, loss_function, camera, point);
+  if (!AddObservations(&problem, bal, Flag(argc, argv, "--bulk") != nullptr, loss)) {
+    std::fprintf(stderr, "unknown --loss=%s\n", loss);
+    return 1;
   }
   if (Flag(argc, argv, "--constant_first_camera")) problem.SetParameterBlockConstant(&bal.cameras[0]);
 

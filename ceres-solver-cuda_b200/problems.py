@@ -64,6 +64,18 @@ COST_TYPES = {
 LOSS_NONE, LOSS_TRIVIAL, LOSS_HUBER, LOSS_CAUCHY = 0, 1, 2, 3
 LOSS_SCALED_HUBER, LOSS_SCALED_CAUCHY, LOSS_SCALED_TRIVIAL = 4, 5, 6
 LOSS_CONVEX_TEST = 7  # test-only user loss rho(s) = s + a s^2 (rho'' > 0)
+# (tests/driver/driver_losses.cu: SnavelyReprojectionError; SoftLOne also on RelativePoseError)
+LOSS_SOFT_L1, LOSS_ARCTAN, LOSS_TOLERANT, LOSS_TUKEY = 8, 9, 10, 11  # (a); Tolerant (a, b)
+LOSS_SCALED_SOFT_L1, LOSS_SCALED_TUKEY = 12, 13  # ScaledLossCUDA<...>(L(a), b)
+LOSS_COMPOSED = 14  # ComposedLossCUDA(ScaledLossCUDA<SoftLOneLossCUDA>(SoftLOne(a), b), Cauchy(a))
+
+# bal_problem(loss=...) names: kind, a, b
+LOSS_BY_NAME = {
+    "none": (LOSS_NONE, 1.0, 0.0), "huber": (LOSS_HUBER, 1.0, 0.0),
+    "cauchy": (LOSS_CAUCHY, 1.0, 0.0), "soft_l1": (LOSS_SOFT_L1, 1.0, 0.0),
+    "arctan": (LOSS_ARCTAN, 1.0, 0.0), "tolerant": (LOSS_TOLERANT, 1.0, 1.0),
+    "tukey": (LOSS_TUKEY, 1.0, 0.0),
+}
 
 # ---- manifold kinds (internal/ceres/manifold.cc, include/ceres/product_manifold.h)
 MANIFOLD_NONE, MANIFOLD_SUBSET, MANIFOLD_QUATERNION, MANIFOLD_EIGEN_QUATERNION = 0, 1, 2, 3
@@ -261,7 +273,7 @@ def bal_problem(num_cameras, num_points, num_observations, seed=1, loss="huber",
     rb_pb = np.empty((nobs, 2), dtype=np.int32)
     rb_pb[:, 0] = npts + cam_of_obs  # argument 0 = camera
     rb_pb[:, 1] = point_of_obs       # argument 1 = point
-    kind = {"none": LOSS_NONE, "huber": LOSS_HUBER, "cauchy": LOSS_CAUCHY}[loss]
+    kind, loss_a, loss_b = LOSS_BY_NAME[loss]
     mk = np.zeros(npts + nc, np.int32)
     mp = np.zeros(npts + nc, np.int32)
     if subset_manifold:  # SubsetManifold(9, {0}) on every camera (BASELINE.json config 4)
@@ -274,8 +286,8 @@ def bal_problem(num_cameras, num_points, num_observations, seed=1, loss="huber",
         pb_size=pb_size, pb_values=pb_values,
         rb_type=np.full(nobs, SNAVELY, np.int32), rb_pb=rb_pb.ravel(), fdata=obs.ravel(),
         pb_constant=const, pb_manifold_kind=mk, pb_manifold_param=mp,
-        rb_loss_kind=np.full(nobs, kind, np.int32), rb_loss_a=np.full(nobs, 1.0),
-        rb_loss_b=np.zeros(nobs), num_eliminate_blocks=npts,
+        rb_loss_kind=np.full(nobs, kind, np.int32), rb_loss_a=np.full(nobs, loss_a),
+        rb_loss_b=np.full(nobs, loss_b), num_eliminate_blocks=npts,
         meta={"workload": f"bal-{nc}x{npts}", "num_cameras": nc, "num_points": npts,
               "num_observations": nobs, "seed": seed})
 
